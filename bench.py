@@ -248,6 +248,12 @@ def run_ours(args):
     ms_total = float(t.item())
     pm, _ = eng.download(out_angles=False)
     refine = eng.exact_argmax_info()
+    if args.dump_outputs:
+        top = None
+        if K:  # every rank takes part in the selection of the K most probable orientations
+            top = eng.top_angles_nccl(K, o_lo, o_hi) if world > 1 else eng.download_top_angles(K)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, pm, top)
 
     # ---- correctness behind the multi-GPU number: the sharded + NCCL-merged result of an orientation prefix
     # against ONE rank evaluating the same prefix alone (bit-identical records expected)
@@ -387,6 +393,19 @@ def run_ours(args):
     eng.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, pm: np.ndarray, top: np.ndarray | None) -> None:
+    """Write what a caller of the timed path receives after its last step, one DIR/<field>.npy per field, so that two
+    builds can be compared output for output on the same seeded inputs: the per-particle records (float64, exact for
+    the integer fields; norm and mu as the float32 they are) and, with WRITE_PROB_ANGLES, the K most probable
+    orientations per particle as top_<field>.npy.  At most 10,000 particles x 10 orientations: a few MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: pm[k].astype(np.float32 if pm.dtype[k] == np.float32 else np.float64) for k in pm.dtype.names}
+    if top is not None:
+        arrays.update({f"top_{k}": top[k].astype(np.float64) for k in ("orient", "forAngles", "ConstAngle")})
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def _mkl_lib() -> str:
@@ -595,7 +614,9 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--steps", type=int, default=2,
+                    help="timed steps of the measurement (the end-to-end leg, which rebuilds every input per step, times "
+                         "min(2, steps) of its own; e2e.steps reports them)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
@@ -605,7 +626,14 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="CPU work budget of one reference sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end leg (profiling runs only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (inputs are seeded: same arguments, "
+                         "same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference arm times the reference binary")
     if args.impl == "reference":
         run_reference(args)
     else:

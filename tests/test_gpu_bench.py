@@ -5,9 +5,11 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from bioem_b200 import api
+from bioem_b200.cases import build_case
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
@@ -37,3 +39,34 @@ def test_bench_line_has_the_contract_keys():
     assert abs(d["roofline"]["frac"] - d["roofline"]["achieved"] / d["roofline"]["peak"]) < 1e-3
     for k in ("sm_mhz", "sm_max_mhz", "reasons"):
         assert k in d["clocks"], k
+
+
+def test_bench_dumps_what_the_last_timed_step_computed(tmp_path):
+    """--dump-outputs: the per-particle records and the WRITE_PROB_ANGLES top-K table of the last timed step, as
+    float32 / float64 .npy files, equal to what the library returns for the same seeded inputs outside bench.py."""
+    if api.lib().bioem_b200_device_count() == 0:
+        pytest.fail("no CUDA device visible: the gpu-marked tests must run on the B200 box")
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "cfg5", "--particles", "8",
+                        "--orientations", "64", "--steps", "2", "--warmup", "1", "--no-cpu-baseline", "--no-e2e",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, cwd=ROOT, timeout=600)
+    assert r.returncode == 0, r.stderr[-800:]
+    got = {p.stem: np.load(p) for p in out.glob("*.npy")}
+    fields = list(api.PROB_MAP_DTYPE.names)
+    assert set(got) == set(fields) | {"top_orient", "top_forAngles", "top_ConstAngle"}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    cd = build_case("cfg5", n_particles=8, n_orient=64)
+    hi, parts = api.inputs_for_case(cd)
+    eng = api.Engine(hi.cfg)
+    try:
+        eng.upload_all(hi, parts)
+        eng.run()
+        pm, _ = eng.download(out_angles=False)
+        top = eng.download_top_angles(cd.case.write_angles)
+    finally:
+        eng.close()
+    for k in fields:
+        np.testing.assert_array_equal(got[k], pm[k])
+    for k in ("orient", "forAngles", "ConstAngle"):
+        np.testing.assert_array_equal(got["top_" + k], top[k])

@@ -214,13 +214,13 @@ def test_host_binary_orientation_grids_and_errors(tmp_path):
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "bioEM_ref")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="reference binary not built (oracle/_ref)")
 @pytest.mark.parametrize("name", ["toy32", "toy36g2"])
 def test_dump_caches_are_interchangeable_with_the_reference(name, tmp_path):
     """--DumpModel / --DumpMaps / --LoadModelDump / --LoadMapDump (reference model.cpp:41-82,676-707,
     map.cpp:44-78): the binary caches have the reference's layout and meaning -- the model as read (before
     the centring, which is redone after loading), the particles as the reader leaves them -- so a cache
-    written by the unmodified reference loads into bioEM_b200 and gives the arrays a direct read gives."""
+    written by the unmodified reference loads into bioEM_b200 and gives the arrays a direct read gives.
+    Without the reference binary, the caches bioEM_b200 writes are the ones loaded back."""
     import subprocess
     from bioem_b200.cases import reference_cli
     exe = _build_host_bin()
@@ -229,12 +229,30 @@ def test_dump_caches_are_interchangeable_with_the_reference(name, tmp_path):
     ref_dir, our_dir, direct, loaded = (tmp_path / d for d in ("ref", "ours", "direct", "loaded"))
     for d in (ref_dir, our_dir, direct, loaded):
         d.mkdir()
-    r = subprocess.run([REF_BIN] + cli + ["--DumpModel", "--DumpMaps", "--PrintCOORDREAD"], cwd=ref_dir,
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
     r = subprocess.run([exe] + cli + ["--DumpModel", "--DumpMaps", "--PrintCOORDREAD"], cwd=our_dir, capture_output=True, text=True,
                        env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(direct)})
     assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
+    if os.path.exists(REF_BIN):
+        r = subprocess.run([REF_BIN] + cli + ["--DumpModel", "--DumpMaps", "--PrintCOORDREAD"], cwd=ref_dir,
+                           capture_output=True, text=True)
+        assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
+        _compare_caches_with_the_reference(cd, ref_dir, our_dir)
+    else:
+        ref_dir = our_dir
+    # load the caches (the REFERENCE's when it is built): same arrays as the direct read (model centred after loading)
+    r = subprocess.run([exe] + cli + ["--LoadModelDump", "--LoadMapDump"], cwd=ref_dir, capture_output=True, text=True,
+                       env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(loaded)})
+    assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
+    p_direct = np.fromfile(direct / "points.bin", dtype=api.MODEL_POINT_DTYPE)
+    p_loaded = np.fromfile(loaded / "points.bin", dtype=api.MODEL_POINT_DTYPE)
+    np.testing.assert_allclose(p_loaded["pos"], p_direct["pos"], rtol=0, atol=2e-6)
+    assert np.array_equal(p_loaded["radius"], p_direct["radius"]) and np.array_equal(p_loaded["density"], p_direct["density"])
+    m_direct = np.fromfile(direct / "maps.bin", dtype=np.float32)
+    m_loaded = np.fromfile(loaded / "maps.bin", dtype=np.float32)
+    np.testing.assert_allclose(m_loaded, m_direct, rtol=0, atol=2.5e-7 * np.abs(m_direct).max())
+
+
+def _compare_caches_with_the_reference(cd, ref_dir, our_dir):
     # COORDREAD (model.cpp:712-740): same lines, the centred coordinates to the last printed digit or one off
     la, lb = (open(d / "COORDREAD").read().split("\n") for d in (ref_dir, our_dir))
     assert len(la) == len(lb) and la[0] == lb[0]
@@ -259,27 +277,17 @@ def test_dump_caches_are_interchangeable_with_the_reference(name, tmp_path):
         assert ma.tobytes() == mb.tobytes()
     else:
         np.testing.assert_allclose(mb, ma, rtol=0, atol=2.5e-7 * np.abs(ma).max())
-    # load the REFERENCE's caches: same arrays as the direct read (model centred after loading)
-    r = subprocess.run([exe] + cli + ["--LoadModelDump", "--LoadMapDump"], cwd=ref_dir, capture_output=True, text=True,
-                       env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(loaded)})
-    assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
-    p_direct = np.fromfile(direct / "points.bin", dtype=api.MODEL_POINT_DTYPE)
-    p_loaded = np.fromfile(loaded / "points.bin", dtype=api.MODEL_POINT_DTYPE)
-    np.testing.assert_allclose(p_loaded["pos"], p_direct["pos"], rtol=0, atol=2e-6)
-    assert np.array_equal(p_loaded["radius"], p_direct["radius"]) and np.array_equal(p_loaded["density"], p_direct["density"])
-    m_direct = np.fromfile(direct / "maps.bin", dtype=np.float32)
-    m_loaded = np.fromfile(loaded / "maps.bin", dtype=np.float32)
-    np.testing.assert_allclose(m_loaded, m_direct, rtol=0, atol=2.5e-7 * np.abs(m_direct).max())
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="reference binary not built (oracle/_ref)")
 @pytest.mark.parametrize("tag,extra,ncol", [("euler", "GRIDPOINTS_ALPHA 4\nGRIDPOINTS_BETA 3\n", 3),
                                             ("quat2", "USE_QUATERNIONS\nGRIDPOINTS_QUATERNION 2\n", 4),
                                             ("quat3", "USE_QUATERNIONS\nGRIDPOINTS_QUATERNION 3\n", 4)])
 def test_orientation_grids_match_the_reference_binary(tag, extra, ncol, tmp_path):
     """Euler / quaternion grid generators (param.cpp:1009-1048,1141-1210) against the unmodified reference:
     with WRITE_PROB_ANGLES = number of orientations its ANG_PROB lists every orientation of the grid (4
-    decimals); the multiset of rows must be the grid bioEM_b200 hands to the library."""
+    decimals); the multiset of rows must be the grid bioEM_b200 hands to the library.  Without the reference binary,
+    the Euler grid is checked against the reference's stored output for the same grid (tests/golden/toy32euler): every
+    orientation it printed must be a point of the grid."""
     import collections
     import subprocess
     exe = _build_host_bin()
@@ -294,6 +302,25 @@ def test_orientation_grids_match_the_reference_binary(tag, extra, ncol, tmp_path
                        env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(hook)})
     assert r.returncode == 0, r.stderr[-400:]
     ang = np.fromfile(hook / "angles.bin", dtype=np.float32).reshape(-1, 4).astype(np.float64)
+
+    def norm(row):  # "-0.0000" and "0.0000" are the same angle
+        return tuple(0.0 if abs(v) < 5e-5 else v for v in row)
+
+    mine = [tuple(float(f"{v:.4f}") for v in a[:ncol]) for a in ang]
+    if not os.path.exists(REF_BIN):
+        if tag != "euler":
+            pytest.skip("reference binary not built (oracle/_ref) and no stored reference output for this grid")
+        from bioem_b200.cases import CASES
+        from bioem_b200.outputs import parse_output_probabilities
+        assert CASES["toy32euler"].euler_grid == (4, 3)
+        gold = os.path.join(ROOT, "tests", "golden", "toy32euler")
+        rows = [tuple(float(x) for x in ln.split()[1:4]) for ln in open(os.path.join(gold, "ANG_PROB")).read().split("\n")
+                if "Separated:" in ln]
+        rows += [tuple(a[:3]) for a in parse_output_probabilities(os.path.join(gold, "Output_Probabilities"), False)["angles"]]
+        assert len(rows) >= 9 and len(mine) == 4 * 3 * 4
+        grid = set(map(norm, mine))
+        assert all(norm(r) in grid for r in rows), sorted(set(map(norm, rows)) - grid)
+        return
     (tmp_path / "p.txt").write_text(common + extra + f"WRITE_PROB_ANGLES {len(ang)}\n")
     r = subprocess.run([REF_BIN] + base, cwd=tmp_path, capture_output=True, text=True)
     assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
@@ -302,19 +329,14 @@ def test_orientation_grids_match_the_reference_binary(tag, extra, ncol, tmp_path
         t = ln.split()
         if len(t) > 6 and t[0] == "0" and "Separated:" in t:
             rows.append(tuple(float(x) for x in t[1:1 + ncol]))
-
-    def norm(row):  # "-0.0000" and "0.0000" are the same angle
-        return tuple(0.0 if abs(v) < 5e-5 else v for v in row)
-
-    mine = [tuple(float(f"{v:.4f}") for v in a[:ncol]) for a in ang]
     assert len(rows) == len(mine)
     assert collections.Counter(map(norm, rows)) == collections.Counter(map(norm, mine))
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="reference binary not built (oracle/_ref)")
 def test_multiple_mrc_list_matches_the_reference_binary(tmp_path):
     """--ReadMRC --ReadMultipleMRC (map.cpp:196-243): a text file naming several MRC stacks; the particles must
-    come out in the reference's order and normalisation (its maps.dump is the witness)."""
+    come out in the reference's order and normalisation (its maps.dump is the witness, when the reference binary is
+    built), and as the single-stack reading of the same images leaves them."""
     import subprocess
     from bioem_b200 import synth
     exe = _build_host_bin()
@@ -328,15 +350,18 @@ def test_multiple_mrc_list_matches_the_reference_binary(tmp_path):
     ref_dir, our_dir, hook = tmp_path / "ref", tmp_path / "ours", tmp_path / "hook"
     for d in (ref_dir, our_dir, hook):
         d.mkdir()
-    r = subprocess.run([REF_BIN] + cli, cwd=ref_dir, capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
     r = subprocess.run([exe] + cli, cwd=our_dir, capture_output=True, text=True,
                        env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(hook)})
     assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
-    a, b = (open(d / "maps.dump", "rb").read() for d in (ref_dir, our_dir))
-    assert len(a) == len(b) and a[:4] == b[:4] and np.frombuffer(a[:4], "<i4")[0] == len(imgs)
-    ma, mb = (np.frombuffer(x[4:], "<f4") for x in (a, b))
-    np.testing.assert_allclose(mb, ma, rtol=0, atol=2.5e-7 * np.abs(ma).max())  # -ffast-math rounding of the reference
+    b = open(our_dir / "maps.dump", "rb").read()
+    assert np.frombuffer(b[:4], "<i4")[0] == len(imgs)
+    if os.path.exists(REF_BIN):
+        r = subprocess.run([REF_BIN] + cli, cwd=ref_dir, capture_output=True, text=True)
+        assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
+        a = open(ref_dir / "maps.dump", "rb").read()
+        assert len(a) == len(b) and a[:4] == b[:4]
+        ma, mb = (np.frombuffer(x[4:], "<f4") for x in (a, b))
+        np.testing.assert_allclose(mb, ma, rtol=0, atol=2.5e-7 * np.abs(ma).max())  # -ffast-math rounding of the reference
     # and the single-stack reading of the same images gives the same particles
     single = tmp_path / "single"
     single.mkdir()
@@ -347,10 +372,10 @@ def test_multiple_mrc_list_matches_the_reference_binary(tmp_path):
     assert open(single / "maps.dump", "rb").read() == b
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="reference binary not built (oracle/_ref)")
 def test_pdb_reader_matches_the_reference_binary(tmp_path):
     """--ReadPDB (model.cpp:85-329,738-844): C-alpha atoms only, residue name -> radius / number of electrons
-    for all 20 residue types, fixed columns; the reference's model.dump is the witness."""
+    for all 20 residue types, fixed columns; the reference's model.dump is the witness when the reference binary is
+    built.  Without it: one point per CA record, at the coordinates of its fixed columns."""
     import subprocess
     exe = _build_host_bin()
     cd = build_case("toy32", str(tmp_path))
@@ -370,23 +395,36 @@ def test_pdb_reader_matches_the_reference_binary(tmp_path):
     ref_dir, our_dir, hook = tmp_path / "ref", tmp_path / "ours", tmp_path / "hook"
     for d in (ref_dir, our_dir, hook):
         d.mkdir()
-    r = subprocess.run([REF_BIN] + cli, cwd=ref_dir, capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
     r = subprocess.run([exe] + cli, cwd=our_dir, capture_output=True, text=True,
                        env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(hook)})
     assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
-    a, b = (open(d / "model.dump", "rb").read() for d in (ref_dir, our_dir))
-    assert len(a) == len(b) and a[4:8] == b[4:8] and np.frombuffer(a[4:8], "<i4")[0] == len(res)
+    b = open(our_dir / "model.dump", "rb").read()
+    assert np.frombuffer(b[4:8], "<i4")[0] == len(res)
+    pb = np.frombuffer(b[8:], "<f4").reshape(-1, 6)
+    ca = np.array([[float(ln[30:38]), float(ln[38:46]), float(ln[46:54])] for ln in lines if ln[12:16] == " CA "],
+                  dtype=np.float32)
+    assert np.array_equal(pb[:, :3], ca)
+    if os.path.exists(REF_BIN):
+        r = subprocess.run([REF_BIN] + cli, cwd=ref_dir, capture_output=True, text=True)
+        assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
+        _compare_model_dumps(open(ref_dir / "model.dump", "rb").read(), b)
+
+
+def _compare_model_dumps(a, b):
+    """model.dump of the reference (a) and of bioEM_b200 (b): same point count, NormDen to the reference's rounding, the
+    same float bits of pos[3], radius and density (column 3 is the unused quat4 of the point struct)"""
+    assert len(a) == len(b) and a[4:8] == b[4:8]
     assert abs(np.frombuffer(a[:4], "<f4")[0] - np.frombuffer(b[:4], "<f4")[0]) <= 4e-7 * np.frombuffer(a[:4], "<f4")[0]
     pa, pb = (np.frombuffer(x[8:], "<f4").reshape(-1, 6) for x in (a, b))
     for col in (0, 1, 2, 4, 5):
         assert pa[:, col].tobytes() == pb[:, col].tobytes(), col
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="reference binary not built (oracle/_ref)")
 def test_mrc_volume_model_reader_matches_the_reference_binary(tmp_path):
     """--ReadModelMRC (model.cpp:332-416, BASELINE configs[3]): one model point per voxel of a mode-2 volume at
-    ((i - nx/2) px, (j - ny/2) px, (k - nz/2) px), radius 2 px, density = voxel; witness: the reference's model.dump."""
+    ((i - nx/2) px, (j - ny/2) px, (k - nz/2) px), radius 2 px, density = voxel; witness: the reference's model.dump
+    when the reference binary is built, and always synth.volume_to_points, the restatement of the reader that the cfg4
+    cases are built with (their oracle results are pinned to the reference's output in tests/golden/cfg4_voxel_slice)."""
     import struct
     import subprocess
     exe = _build_host_bin()
@@ -406,14 +444,17 @@ def test_mrc_volume_model_reader_matches_the_reference_binary(tmp_path):
     ref_dir, our_dir, hook = tmp_path / "ref", tmp_path / "ours", tmp_path / "hook"
     for d in (ref_dir, our_dir, hook):
         d.mkdir()
-    r = subprocess.run([REF_BIN] + cli, cwd=ref_dir, capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
     r = subprocess.run([exe] + cli, cwd=our_dir, capture_output=True, text=True,
                        env={**os.environ, "BIOEM_B200_DUMP_INPUTS": str(hook)})
     assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
-    a, b = (open(d / "model.dump", "rb").read() for d in (ref_dir, our_dir))
-    assert len(a) == len(b) and a[4:8] == b[4:8] and np.frombuffer(a[4:8], "<i4")[0] == nx * ny * nz
-    assert abs(np.frombuffer(a[:4], "<f4")[0] - np.frombuffer(b[:4], "<f4")[0]) <= 4e-7 * np.frombuffer(a[:4], "<f4")[0]
-    pa, pb = (np.frombuffer(x[8:], "<f4").reshape(-1, 6) for x in (a, b))
-    for col in (0, 1, 2, 4, 5):
-        assert pa[:, col].tobytes() == pb[:, col].tobytes(), col
+    b = open(our_dir / "model.dump", "rb").read()
+    assert np.frombuffer(b[4:8], "<i4")[0] == nx * ny * nz
+    pb = np.frombuffer(b[8:], "<f4").reshape(-1, 6)
+    from bioem_b200 import synth
+    want = synth.volume_to_points(vol.reshape(-1).reshape(nx, ny, nz), cd.case.pixel_size).astype(np.float32)
+    for col, wcol in ((0, 0), (1, 1), (2, 2), (4, 3), (5, 4)):
+        assert np.array_equal(pb[:, col], want[:, wcol]), col
+    if os.path.exists(REF_BIN):
+        r = subprocess.run([REF_BIN] + cli, cwd=ref_dir, capture_output=True, text=True)
+        assert r.returncode == 0, r.stdout[-400:] + r.stderr[-400:]
+        _compare_model_dumps(open(ref_dir / "model.dump", "rb").read(), b)

@@ -1,5 +1,5 @@
 import os,sys,time
-sys.path.insert(0,'/root/repo')
+sys.path.insert(0,os.path.join(os.path.dirname(os.path.abspath(__file__)),'..'))
 import torch
 from bioem_b200 import api
 from bioem_b200.cases import build_case
