@@ -57,7 +57,7 @@ EXPORTS = [
     "bioem_b200_top_angles_nccl", "bioem_b200_set_kernel_timing", "bioem_b200_out_of_frame",
     "bioem_b200_exact_argmax_info", "bioem_b200_cached_product", "bioem_b200_stream", "bioem_b200_device_angles", "bioem_b200_stats",
     "bioem_b200_kernel_time", "bioem_b200_debug_projection", "bioem_b200_debug_convolved",
-    "bioem_b200_debug_correlation", "bioem_b200_debug_particle",
+    "bioem_b200_debug_correlation", "bioem_b200_debug_run_values", "bioem_b200_debug_particle",
     "bioem_b200_host_defocus_to_phase", "bioem_b200_host_ctf_table", "bioem_b200_host_psf_kernels",
     "bioem_b200_host_volu",
     "bioem_b200_host_model_prepare", "bioem_b200_host_normalise_map",
@@ -129,6 +129,7 @@ def lib():
     L.bioem_b200_debug_projection.argtypes = [vp, C.c_int, fp]
     L.bioem_b200_debug_convolved.argtypes = [vp, C.c_int, C.c_int, fp, fp, fp]
     L.bioem_b200_debug_correlation.argtypes = [vp, C.c_int, C.c_int, C.c_int, fp, C.POINTER(C.c_int)]
+    L.bioem_b200_debug_run_values.argtypes = [vp, C.c_int, C.c_int, fp]
     L.bioem_b200_debug_particle.argtypes = [vp, C.c_int, fp, fp, fp]
     L.bioem_b200_host_defocus_to_phase.argtypes = [C.c_float, C.c_float, C.c_float, fp, fp, fp, fp]
     L.bioem_b200_host_defocus_to_phase.restype = None
@@ -426,14 +427,26 @@ class Engine:
              "debug_convolved")
         return out, s.value, ss.value
 
-    def debug_correlation(self, o: int, c: int, m: int) -> np.ndarray:
+    def _window_edge(self) -> int:
         d, g = self.cfg.maxDisplaceCenter, self.cfg.GridSpaceCenter
-        nw = d // g + 1 + (d + g - 1) // g  # Algo 1's window (bioem_algorithm.h:156-197), quirk Q3
+        return d // g + 1 + (d + g - 1) // g  # Algo 1's window (bioem_algorithm.h:156-197), quirk Q3
+
+    def debug_correlation(self, o: int, c: int, m: int) -> np.ndarray:
+        nw = self._window_edge()
         out = np.zeros(nw * nw, dtype=np.float32)
         nv = C.c_int()
         _chk(lib().bioem_b200_debug_correlation(self._h, int(o), int(c), int(m), _fp(out), C.byref(nv)),
              "debug_correlation")
         return out.reshape(nw, nw)
+
+    def run_capture(self, o_begin: int = 0, o_end: int | None = None) -> np.ndarray:
+        """run(o_begin, o_end), returning every correlation window it computed: [o_end - o_begin, C, M, nw, nw]
+        (each window as debug_correlation returns it)."""
+        o_end = self.O if o_end is None else o_end
+        nw = self._window_edge()
+        out = np.zeros((max(0, o_end - o_begin), self.C, self.M, nw, nw), dtype=np.float32)
+        _chk(lib().bioem_b200_debug_run_values(self._h, int(o_begin), int(o_end), _fp(out)), "debug_run_values")
+        return out
 
     def debug_particle(self, m: int):
         n = self.cfg.NumberPixels

@@ -1154,7 +1154,9 @@ static int run_generic_batch(bioem_b200_context *h, int o0, int OBcur)
   return BIOEM_B200_OK;
 }
 
-int bioem_b200_run(bioem_b200_handle h, int oBegin, int oEnd)
+// run() for orientations [oBegin, oEnd); capture != nullptr (inspection): every correlation value lCC/N^2 of the range
+// is copied out as well, capture[o - oBegin][c][m][nw*nw], in the window order of debug_correlation
+static int run_range(bioem_b200_context *h, int oBegin, int oEnd, float *capture)
 {
   if (!h)
     return fail(BIOEM_B200_ERR_INVALID, "run: null handle");
@@ -1178,6 +1180,18 @@ int bioem_b200_run(bioem_b200_handle h, int oBegin, int oEnd)
     rc = run_front(h, o0, OBcur);
     if (rc)
       return rc;
+    // capture: the batch's windows land in a temp (fused kernel) or in d_values (direct-DFT path), prefilled with
+    // 0xFF bytes -- a NaN -- so that an entry the kernel does not write shows up
+    const size_t ncap = capture ? (size_t) OBcur * h->C * h->M * h->nw * h->nw : 0;
+    DevTmp t_cap(h);
+    float *d_cap = nullptr;
+    if (capture)
+    {
+      if (!h->generic)
+        RC(t_cap.alloc(sizeof(float) * ncap));
+      d_cap = h->generic ? h->d_values : t_cap.as<float>();
+      CU(cudaMemsetAsync(d_cap, 0xFF, sizeof(float) * ncap, h->stream));
+    }
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (h->time_kernels)
     {
@@ -1195,6 +1209,8 @@ int bioem_b200_run(bioem_b200_handle h, int oBegin, int oEnd)
     }
     LikParams lp;
     fill_lik_params(h, lp, o0, OBcur);
+    if (capture && !h->generic)
+      lp.dbg_values = d_cap;
     const int NG = (OBcur + h->OG - 1) / h->OG;
     if (h->generic)
     {
@@ -1210,6 +1226,12 @@ int bioem_b200_run(bioem_b200_handle h, int oBegin, int oEnd)
       h->lik_events.emplace_back(e0, e1);
     }
     h->lik_launches += 1;
+    if (capture)
+    {
+      CU(cudaMemcpyAsync(capture + (size_t) (o0 - oBegin) * h->C * h->M * h->nw * h->nw, d_cap, sizeof(float) * ncap,
+                         cudaMemcpyDeviceToHost, h->stream));
+      CU(cudaStreamSynchronize(h->stream));
+    }
     if (h->generic)
       continue;
     merge_partials_kernel<<<(h->M + 127) / 128, 128, 0, h->stream>>>(h->d_partials, NG, h->M, h->d_state);
@@ -1220,6 +1242,8 @@ int bioem_b200_run(bioem_b200_handle h, int oBegin, int oEnd)
   }
   return BIOEM_B200_OK;
 }
+
+int bioem_b200_run(bioem_b200_handle h, int oBegin, int oEnd) { return run_range(h, oBegin, oEnd, nullptr); }
 
 // Exact first-of-ties displacement for the arg-max record of every particle (see exact_argmax_kernel): the
 // winning (orientation, CTF) of each particle is evaluated once more by the fused kernel with its correlation
@@ -1869,6 +1893,13 @@ int bioem_b200_debug_correlation(bioem_b200_handle h, int o, int c, int m, float
   if (nvalues)
     *nvalues = (int) nv;
   return BIOEM_B200_OK;
+}
+
+int bioem_b200_debug_run_values(bioem_b200_handle h, int oBegin, int oEnd, float *values_out)
+{
+  if (!values_out)
+    return fail(BIOEM_B200_ERR_INVALID, "debug_run_values: null output");
+  return run_range(h, oBegin, oEnd, values_out);
 }
 
 int bioem_b200_debug_particle(bioem_b200_handle h, int m, float *fft_out, float *sum, float *sumsq)

@@ -236,6 +236,10 @@ int bioem_b200_debug_convolved(bioem_b200_handle h, int iOrient, int iConv, floa
  * in doRefMapFFT enumeration order (reference bioem_algorithm.h:156-197) */
 int bioem_b200_debug_correlation(bioem_b200_handle h, int iOrient, int iConv, int iMap, float *values_out,
                                  int *nValues);
+/* run(h, oBegin, oEnd) -- same batching, kernel mode and launch grid, the running state accumulates as there, so
+ * download() afterwards is valid -- and every correlation value lCC/N^2 it computes, written to
+ * values_out[(o - oBegin) * nCtf * nMaps + c * nMaps + m][nValues] in the order of debug_correlation.  Synchronous. */
+int bioem_b200_debug_run_values(bioem_b200_handle h, int oBegin, int oEnd, float *values_out);
 /* particle spectrum in the reference layout + its sums */
 int bioem_b200_debug_particle(bioem_b200_handle h, int iMap, float *fft_out, float *sum, float *sumsq);
 

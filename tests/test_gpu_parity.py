@@ -18,6 +18,7 @@ from bioem_b200 import api
 from bioem_b200.cases import build_case
 from bioem_b200.outputs import parse_output_probabilities
 from oracle import pyoracle
+from tests import likmodel
 
 pytestmark = pytest.mark.gpu
 
@@ -107,8 +108,7 @@ def test_particle_precompute_matches_oracle(setups, name):
 
 def _window(P):
     c = P.case
-    N, maxd, G = c.n_pixels, c.max_disp, c.grid_space
-    return list(range(0, maxd + 1, G)) + list(range(N - maxd, N, G))
+    return list(likmodel.window(c.n_pixels, c.max_disp, c.grid_space))
 
 
 @pytest.mark.parametrize("name", ["toy32", "toy32g2odd", "toy32g3", "toy36g2", "toy64", "cfg1", "cfg2_slice", "cfg4_slice",
@@ -507,27 +507,14 @@ def test_out_of_frame_points_are_counted(setups):
     assert eng2.out_of_frame()[1] == 0
 
 
-def _fma32(a, b, c):
-    """float fma: the product of two floats is exact in double, one rounding to double, one to float"""
-    return (a.astype(np.float64) * np.float64(b) + c.astype(np.float64)).astype(np.float32)
-
-
 def _host_first_of_ties(eng, hi, parts_sum, o, c, m, prior):
     """The reference's rule applied on the host to the GPU's own correlation window of one likelihood:
     firstele in FP32 (bioem_algorithm.h:29-36; with the one multiply-add the kernel fuses), logpro in double,
     narrowed to float (:84), first maximum in enumeration order (:96)."""
-    f32 = np.float32
-    v = eng.debug_correlation(o, c, m).astype(np.float32).ravel()
+    v = eng.debug_correlation(o, c, m).ravel()
     _, sC, ssC = eng.debug_convolved(o, c)
     sR, ssR = parts_sum
-    sC, ssC, sR, ssR = f32(sC), f32(ssC), f32(sR), f32(ssR)
-    Nt = f32(hi.cfg.Ntotpi)
-    fe = _fma32(ssR * ssC - v * v, Nt, (f32(2.0) * sR * sC) * v) - (ssR * sC) * sC - (sR * sR) * ssC
-    assert fe.dtype == np.float32
-    fl = ssC * Nt - sC * sC
-    a = (3.0 - float(Nt)) * 0.5
-    bterm = (float(Nt) * 0.5 - 2.0) * np.log(float(Nt - f32(2.0)) * float(fl)) - prior
-    lp = (a * np.log(fe.astype(np.float64)) + bterm).astype(np.float32)
+    lp = likmodel.logpro(v, sR, ssR, sC, ssC, hi.cfg.Ntotpi, prior).astype(np.float32)
     return int(np.argmax(lp)), lp  # argmax returns the FIRST maximum
 
 
@@ -561,7 +548,7 @@ def test_exact_first_of_ties_displacement():
         ties = []
         for m in range(parts.shape[0]):
             _, sR, ssR = e.debug_particle(m)
-            first, lp = _host_first_of_ties(e, hi, (sR, ssR), 0, 0, m, _prior(hi, one_ctf[1][0]))
+            first, lp = _host_first_of_ties(e, hi, (sR, ssR), 0, 0, m, likmodel.prior(hi, one_ctf[1][0]))
             nw = int(round(np.sqrt(lp.size)))
             wx, wy = divmod(first, nw)
             npos = hi.cfg.maxDisplaceCenter // hi.cfg.GridSpaceCenter + 1
@@ -575,18 +562,6 @@ def test_exact_first_of_ties_displacement():
         assert ev == parts.shape[0] and bad == 0
     finally:
         e.close()
-
-
-def _prior(hi, ctfparam):
-    """prior term of calc_logpro in CTF mode (bioem_algorithm.h:49-56) with the library's (and the reference's)
-    arithmetic: products of floats are float products, the divisions run in double"""
-    f32 = np.float32
-    amp, pha, env = (f32(x) for x in ctfparam[:3])
-    c = hi.cfg
-    dp, da = pha - f32(c.Priordefcent), amp - f32(c.Priorampcent)
-    return (float(env * env) / 2. / float(f32(c.sigmaPriorbctf)) / float(f32(c.sigmaPriorbctf))
-            - float(dp * dp) / 2. / float(f32(c.sigmaPriordefo)) / float(f32(c.sigmaPriordefo))
-            - float(da * da) / 2. / float(f32(c.sigmaPrioramp)) / float(f32(c.sigmaPrioramp)))
 
 
 def test_exact_ties_between_ctfs_orientations_groups_and_launches(monkeypatch, setups):
