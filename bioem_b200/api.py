@@ -56,7 +56,7 @@ EXPORTS = [
     "bioem_b200_nccl_unique_id", "bioem_b200_nccl_init", "bioem_b200_nccl_attach", "bioem_b200_nccl_comm", "bioem_b200_merge_nccl",
     "bioem_b200_top_angles_nccl", "bioem_b200_set_kernel_timing", "bioem_b200_out_of_frame",
     "bioem_b200_exact_argmax_info", "bioem_b200_cached_product", "bioem_b200_stream", "bioem_b200_device_angles", "bioem_b200_stats",
-    "bioem_b200_kernel_time", "bioem_b200_debug_projection", "bioem_b200_debug_convolved",
+    "bioem_b200_kernel_time", "bioem_b200_render_maps", "bioem_b200_debug_projection", "bioem_b200_debug_convolved",
     "bioem_b200_debug_correlation", "bioem_b200_debug_run_values", "bioem_b200_debug_particle",
     "bioem_b200_host_defocus_to_phase", "bioem_b200_host_ctf_table", "bioem_b200_host_psf_kernels",
     "bioem_b200_host_volu",
@@ -126,6 +126,7 @@ def lib():
     L.bioem_b200_device_angles.restype = vp
     L.bioem_b200_stats.argtypes = [vp, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.bioem_b200_kernel_time.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_longlong)]
+    L.bioem_b200_render_maps.argtypes = [vp, vp, C.c_int, fp]
     L.bioem_b200_debug_projection.argtypes = [vp, C.c_int, fp]
     L.bioem_b200_debug_convolved.argtypes = [vp, C.c_int, C.c_int, fp, fp, fp]
     L.bioem_b200_debug_correlation.argtypes = [vp, C.c_int, C.c_int, C.c_int, fp, C.POINTER(C.c_int)]
@@ -411,6 +412,20 @@ class Engine:
         t, n = C.c_double(), C.c_longlong()
         _chk(lib().bioem_b200_kernel_time(self._h, C.byref(t), C.byref(n)), "kernel_time")
         return t.value, n.value
+
+    # ---- calculated images
+    def render_maps(self, records: np.ndarray) -> np.ndarray:
+        """float32 [n, N, N]: the calculated image each record names (its orientation, CTF, displacement, norm and
+        mu), in the layout of the particles given to upload_particles; records is a PROB_MAP_DTYPE array, e.g. the
+        first result of download(), whose maps are then every particle's best fit."""
+        r = np.ascontiguousarray(records)
+        if r.dtype != PROB_MAP_DTYPE:
+            raise TypeError(f"render_maps: records must be of PROB_MAP_DTYPE, not {r.dtype}")
+        r = r.reshape(-1)
+        n = self.cfg.NumberPixels
+        out = np.zeros((len(r), n, n), dtype=np.float32)
+        _chk(lib().bioem_b200_render_maps(self._h, r.ctypes.data, len(r), _fp(out)), "render_maps")
+        return out
 
     # ---- inspection
     def debug_projection(self, o: int) -> np.ndarray:

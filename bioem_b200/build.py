@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libbioem_b200.so")
 SOURCES = ["bioem_b200.cu", "host_prep.cpp"]
-HEADERS = ["bioem_kernels.cuh", "generic_kernels.cuh", "fft_regs.cuh", "lik_instance.inl",
+HEADERS = ["bioem_kernels.cuh", "generic_kernels.cuh", "render_kernels.cuh", "fft_regs.cuh", "lik_instance.inl",
            os.path.join("..", "..", "include", "bioem_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 CFLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

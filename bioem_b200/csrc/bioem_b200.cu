@@ -2,6 +2,7 @@
 #include "../../include/bioem_b200.h"
 #include "bioem_kernels.cuh"
 #include "generic_kernels.cuh"
+#include "render_kernels.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -456,6 +457,45 @@ static cudaError_t do_lik(int N, const LikParams &p, int nblocks, int maxD, cuda
 #define X(n)                                                                                              \
   case n:                                                                                                 \
     return bioem_lik_launch_##n(&p, nblocks, maxD, s);
+    BIOEM_SIZES(X)
+#undef X
+  }
+  return cudaErrorInvalidValue;
+}
+// calculated images of a batch (render_kernels.cuh): conv spectra -> scratch [item][N][N/2+1] -> out [item][N][N]
+template <int N>
+static cudaError_t launch_render(const float4 *convs, const RenderItem *items, const float2 *tw_inv, float2 *scratch, float *out,
+                                 int nitems, cudaStream_t s)
+{
+  using L = Lay<N>;
+  dim3 g1((N / 2 + 1 + L::FKC - 1) / L::FKC, nitems);
+  const size_t smem1 = sizeof(float2) * (size_t) (L::FKC * N + N);
+  cudaError_t e = cudaFuncSetAttribute(render_cols_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem1);
+  if (e != cudaSuccess)
+    return e;
+  render_cols_kernel<N><<<g1, NT, smem1, s>>>(convs, items, tw_inv, scratch);
+  dim3 g2((N / 2 + L::PC - 1) / L::PC, nitems);
+  render_rows_kernel<N><<<g2, NT, 0, s>>>(scratch, items, tw_inv, out);
+  return cudaGetLastError();
+}
+static cudaError_t do_render(int N, const float4 *convs, const RenderItem *items, const float2 *tw_inv, float2 *scratch, float *out,
+                             int nitems, cudaStream_t s)
+{
+  if (is_generic(N))
+  {
+    gen_render_cols_kernel<<<dim3(N, nitems), 256, (size_t) N * sizeof(float2), s>>>(
+        reinterpret_cast<const float2 *>(convs), 2 * map4_generic(N), items, tw_inv, N, scratch);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess)
+      return e;
+    gen_render_rows_kernel<<<dim3(N, nitems), 256, (size_t) (N + N / 2 + 1) * sizeof(float2), s>>>(scratch, items, tw_inv, N, out);
+    return cudaGetLastError();
+  }
+  switch (N)
+  {
+#define X(n)                                                                                              \
+  case n:                                                                                                 \
+    return launch_render<n>(convs, items, tw_inv, scratch, out, nitems, s);
     BIOEM_SIZES(X)
 #undef X
   }
@@ -1061,8 +1101,10 @@ int bioem_b200_reset(bioem_b200_handle h)
 }
 
 // stages 1 + 2 for orientations [o0, o0+OBcur) into the batch buffers
+// (conv_dst: where the convolved spectra go when want_conv is set, instead of the batch buffer -- render_maps in
+// cached-product mode, whose batch buffer holds one orientation's worth)
 static int run_front(bioem_b200_context *h, int o0, int OBcur, const float4 *angles = nullptr, const int4 *sel = nullptr,
-                     int nsel = 0, bool want_conv = false)
+                     int nsel = 0, bool want_conv = false, float4 *conv_dst = nullptr)
 {
   const int N = h->N;
   ProjParams pp;
@@ -1089,6 +1131,8 @@ static int run_front(bioem_b200_context *h, int o0, int OBcur, const float4 *ang
   CU(cudaGetLastError());
   CU(do_fft2d(N, h->d_proj, h->d_tempden, h->nbands, h->NormDen, h->d_tw_fwd, h->d_scratch, h->d_projfft, OBcur, h->stream));
   float4 *conv = (h->zmode && !want_conv) ? nullptr : h->d_conv; // (want_conv in cached-product mode: OBcur == 1)
+  if (want_conv && conv_dst)
+    conv = conv_dst;
   CU(do_conv(N, h->d_projfft, h->d_ctf, h->d_prior, conv, h->d_cpar, h->C, OBcur, h->cfg.Ntotpi, h->stream, sel, nsel));
   h->launches += 4;
   return BIOEM_B200_OK;
@@ -1360,6 +1404,129 @@ int bioem_b200_download(bioem_b200_handle h, bioem_b200_prob_map *maps_out, bioe
   if (angles_out && h->cfg.writeAngles && h->d_angtab)
     CU(cudaMemcpyAsync(angles_out, h->d_angtab, sizeof(ProbAngleOut) * (size_t) h->O * h->M, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
+  return BIOEM_B200_OK;
+}
+
+// Calculated images of arbitrary records (bioem_b200.h).  Records are sorted by orientation and taken in batches of
+// at most OB distinct orientations and OB * C images, as the exact arg-max pass does: every distinct orientation is
+// projected once into the batch buffers (a private orientation list, no out-of-frame counting), each image's conv
+// spectrum is formed by the selection path of the conv kernel (a slot per image; on the direct-DFT path every CTF
+// of the batch's orientations), then transformed back and copied out.  Nothing of the running state is touched.
+int bioem_b200_render_maps(bioem_b200_handle h, const bioem_b200_prob_map *records, int n, float *maps_out)
+{
+  if (!h)
+    return fail(BIOEM_B200_ERR_INVALID, "render_maps: null handle");
+  if (n < 0)
+    return fail(BIOEM_B200_ERR_INVALID, "render_maps: negative record count " + std::to_string(n));
+  if (n > 0 && (!records || !maps_out))
+    return fail(BIOEM_B200_ERR_INVALID, "render_maps: null records or output");
+  if (h->A <= 0 || h->O <= 0 || h->C <= 0 || (int) h->h_angles.size() != h->O)
+    return fail(BIOEM_B200_ERR_STATE, "render_maps: model, orientations and CTF table must be uploaded first");
+  const int N = h->N;
+  for (int i = 0; i < n; i++)
+  {
+    const bioem_b200_prob_map &r = records[i];
+    if (r.max_prob_orient < 0 || r.max_prob_orient >= h->O)
+      return fail(BIOEM_B200_ERR_INVALID, "render_maps: record " + std::to_string(i) + ": orientation " +
+                                              std::to_string(r.max_prob_orient) + " out of range [0, " + std::to_string(h->O) + ")");
+    if (r.max_prob_conv < 0 || r.max_prob_conv >= h->C)
+      return fail(BIOEM_B200_ERR_INVALID, "render_maps: record " + std::to_string(i) + ": CTF " + std::to_string(r.max_prob_conv) +
+                                              " out of range [0, " + std::to_string(h->C) + ")");
+    if (r.max_prob_cent_x <= -N || r.max_prob_cent_x >= N || r.max_prob_cent_y <= -N || r.max_prob_cent_y >= N)
+      return fail(BIOEM_B200_ERR_INVALID, "render_maps: record " + std::to_string(i) + ": displacement (" +
+                                              std::to_string(r.max_prob_cent_x) + ", " + std::to_string(r.max_prob_cent_y) +
+                                              ") not inside (-" + std::to_string(N) + ", " + std::to_string(N) + ")");
+  }
+  if (n == 0)
+    return BIOEM_B200_OK;
+  CU(cudaSetDevice(h->device));
+  RC(ensure_batch(h));
+  // (the front end counts its launches; stats() describes run() and stays as it was)
+  struct KeepLaunches
+  {
+    bioem_b200_context *h;
+    long long v;
+    ~KeepLaunches() { h->launches = v; }
+  } keep{h, h->launches};
+  std::vector<int> order((size_t) n);
+  for (int i = 0; i < n; i++)
+    order[i] = i;
+  std::stable_sort(order.begin(), order.end(),
+                   [&](int a, int b) { return records[a].max_prob_orient < records[b].max_prob_orient; });
+  // images per batch: OB * C conv slots, and the 65535 grid rows of the kernels
+  const int cap = (int) std::min<long long>({(long long) h->OB * h->C, (long long) n, 65535LL});
+  const size_t n2 = (size_t) N * N;
+  DevTmp t_out(h), t_scr(h), t_items(h), t_sel(h), t_ang(h), t_conv(h);
+  RC(t_out.alloc(sizeof(float) * n2 * cap));
+  RC(t_scr.alloc(sizeof(float2) * (size_t) N * (N / 2 + 1) * cap));
+  RC(t_items.alloc(sizeof(RenderItem) * cap));
+  RC(t_sel.alloc(sizeof(int4) * cap));
+  RC(t_ang.alloc(sizeof(float4) * h->OB));
+  // the fused path's conv spectra: the batch buffer holds OB * C of them, except in cached-product mode (one
+  // orientation's worth)
+  float4 *convs = h->d_conv;
+  if (!h->generic && h->zmode)
+  {
+    RC(t_conv.alloc(sizeof(float4) * h->map4 * cap));
+    convs = t_conv.as<float4>();
+  }
+  size_t pos = 0;
+  while (pos < order.size())
+  {
+    std::vector<float4> ang;
+    std::vector<int4> sel;
+    std::vector<RenderItem> items;
+    const size_t first = pos;
+    int last = -1;
+    while (pos < order.size())
+    {
+      const bioem_b200_prob_map &r = records[order[pos]];
+      if ((r.max_prob_orient != last && (int) ang.size() == h->OB) || (int) items.size() == cap)
+        break;
+      if (r.max_prob_orient != last)
+      {
+        ang.push_back(h->h_angles[r.max_prob_orient]);
+        last = r.max_prob_orient;
+      }
+      const int ob = (int) ang.size() - 1;
+      RenderItem it;
+      it.slot = h->generic ? ob * h->C + r.max_prob_conv : (int) items.size();
+      it.sx = (r.max_prob_cent_x + N) % N;
+      it.sy = (r.max_prob_cent_y + N) % N;
+      it.norm = r.max_prob_norm;
+      it.mu = r.max_prob_mu;
+      sel.push_back(make_int4(order[pos], ob, r.max_prob_conv, 0));
+      items.push_back(it);
+      pos++;
+    }
+    const int ni = (int) items.size();
+    // output slots in ascending record order: consecutive records land next to each other (all of them, when the
+    // whole call fits one batch) and go back to the caller in one copy per run
+    std::vector<int> recs(order.begin() + first, order.begin() + pos);
+    std::sort(recs.begin(), recs.end());
+    for (int b = 0; b < ni; b++)
+      items[b].out = (int) (std::lower_bound(recs.begin(), recs.end(), order[first + b]) - recs.begin());
+    CU(cudaMemcpyAsync(t_ang.p, ang.data(), sizeof(float4) * ang.size(), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(t_items.p, items.data(), sizeof(RenderItem) * ni, cudaMemcpyHostToDevice, h->stream));
+    if (h->generic) // (no selection path here: every CTF of the batch's orientations, slot ob * C + c)
+      RC(run_front(h, 0, (int) ang.size(), t_ang.as<float4>()));
+    else
+    {
+      CU(cudaMemcpyAsync(t_sel.p, sel.data(), sizeof(int4) * ni, cudaMemcpyHostToDevice, h->stream));
+      RC(run_front(h, 0, (int) ang.size(), t_ang.as<float4>(), t_sel.as<int4>(), ni, true, convs));
+    }
+    CU(do_render(N, convs, t_items.as<RenderItem>(), h->d_tw_inv, t_scr.as<float2>(), t_out.as<float>(), ni, h->stream));
+    for (int b = 0; b < ni;)
+    {
+      int e = b + 1;
+      while (e < ni && recs[e] == recs[e - 1] + 1)
+        e++;
+      CU(cudaMemcpyAsync(maps_out + (size_t) recs[b] * n2, t_out.as<float>() + (size_t) b * n2, sizeof(float) * n2 * (e - b),
+                         cudaMemcpyDeviceToHost, h->stream));
+      b = e;
+    }
+    CU(cudaStreamSynchronize(h->stream)); // the host vectors of this batch go out of scope
+  }
   return BIOEM_B200_OK;
 }
 

@@ -22,6 +22,7 @@ struct Options // reference bioem.cpp:193-224
   bool dumpMaps = false, loadMapDump = false, dumpModel = false, loadModelDump = false;
   bool printCoordRead = false;
   int gpus = 0; // extension: number of GPUs of this box to use (0 = all visible)
+  std::string bestmapsfile; // extension: --WriteBestMaps, every particle's best-fit calculated map (MRC stack)
 };
 
 struct Params // reference bioem_param after readParameters + CalculateGridsParam + CalculateRefCTF
@@ -61,6 +62,9 @@ void read_model(const Options &o, const Params &p, std::vector<bioem_b200_model_
 void read_particles(const Options &o, const Params &p, std::vector<float> &maps, int &nMaps, bool &rawMRC);
 // what the reference's MRC reader does to a raw stack, on the host (for --DumpMaps and the test hook)
 void mrc_host_ingest(const Params &p, std::vector<float> &maps, int nMaps);
+// maps: n x N x N (the layout of the particles handed to the library) -> MRC mode-2 stack that read_particles with
+// --ReadMRC and NO_MAP_NORM reads back to the same arrays
+void write_mrc_stack(const std::string &file, const float *maps, int N, int n);
 // cand: WRITE_PROB_ANGLES candidates, nMaps x nCand rows in ascending orientation order (orient -1 = unused): the
 // per-GPU lists of most probable orientations selected on the device (bioem_b200_download_top_angles)
 void write_outputs(const Options &o, const Params &p, const bioem_b200_config &cfg,

@@ -3,6 +3,7 @@
 //   bioEM_b200 --Modelfile m --Particlesfile p --Inputfile i [--ReadOrientation o] [--ReadPDB]
 //              [--ReadModelMRC] [--ReadMRC] [--ReadMultipleMRC] [--DumpMaps] [--LoadMapDump]
 //              [--DumpModel] [--LoadModelDump] [--PrintCOORDREAD] [--OutputFile f] [--Gpus n]
+//              [--WriteBestMaps f]
 //
 // Flow = the reference's main.cpp:34-140 / bioem::configure / bioem::run with the main loop
 // (bioem.cpp:763-891) replaced by bioem_b200_run on every GPU of the box: the orientation grid is
@@ -342,11 +343,20 @@ int main(int argc, char **argv)
       });
     }
   }
+  // --WriteBestMaps: the merged records rendered on GPU 0 (its handle holds every input)
+  std::vector<float> bestmaps;
+  if (!opt.bestmapsfile.empty())
+  {
+    bestmaps.resize((size_t) nMaps * par.N * par.N);
+    B200(bioem_b200_render_maps(handles[0], pm.data(), nMaps, bestmaps.data()));
+  }
   for (int g = 0; g < ndev; g++)
     bioem_b200_destroy(handles[g]);
   const auto t2 = std::chrono::steady_clock::now();
 
   write_outputs(opt, par, cfg, pm, cand, nCand, nMaps);
+  if (!opt.bestmapsfile.empty())
+    write_mrc_stack(opt.bestmapsfile, bestmaps.data(), par.N, nMaps);
   const auto t3 = std::chrono::steady_clock::now();
   auto sec = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
     return std::chrono::duration<double>(b - a).count();

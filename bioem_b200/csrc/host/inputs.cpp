@@ -2,6 +2,7 @@
 // Behaviour (keywords, defaults, error conditions, file layouts) follows the reference files cited
 // at each function; the code is this project's own.
 #include "bioem_host.hpp"
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -53,6 +54,11 @@ static void usage()
          "  --PrintCOORDREAD       (Optional) Print model coordinates\n"
          "  --OutputFile arg       (Optional) For changing the outputfile name\n"
          "  --Gpus arg             (Extension) number of GPUs of this box to use (default: all)\n"
+         "  --WriteBestMaps arg    (Extension) write every particle's best-fit calculated map (orientation, CTF,\n"
+         "                         displacement, normalisation and offset of its Maximizing Param line) to this\n"
+         "                         file, one MRC mode-2 stack that --ReadMRC with NO_MAP_NORM reads back as the\n"
+         "                         rendered images.  Not the reference's --PrintBestCalMap: its parameter keywords,\n"
+         "                         BESTMAP text format and noise option are not reproduced\n"
          "  --help                 (Optional) Produce help message\n\n");
 }
 
@@ -103,6 +109,8 @@ void parse_options(int argc, char **argv, Options &o)
       o.outfile = need();
     else if (a == "Gpus")
       o.gpus = atoi(need().c_str());
+    else if (a == "WriteBestMaps")
+      o.bestmapsfile = need();
     else if (a == "ReadPDB")
       o.readPDB = true;
     else if (a == "ReadModelMRC")
@@ -620,6 +628,54 @@ static void read_mrc_floats(FILE *f, float *dst, size_t n, bool swap, const char
       u = bswap32(u);
       memcpy(&dst[i], &u, 4);
     }
+}
+
+// --WriteBestMaps: maps[i][x][y] as one mode-2 stack, stored as the reader expects it (read_particles with --ReadMRC
+// stores file[j*N + i] at maps[i*N + j], so the file holds each image transposed)
+void write_mrc_stack(const std::string &file, const float *maps, int N, int n)
+{
+  int w[256];
+  memset(w, 0, sizeof(w));
+  w[0] = N; // nc, nr, ns
+  w[1] = N;
+  w[2] = n;
+  w[3] = 2; // mode: 32-bit float
+  w[7] = N; // mx, my, mz
+  w[8] = N;
+  w[9] = 1;
+  const float cell[6] = {(float) N, (float) N, 1.f, 90.f, 90.f, 90.f};
+  memcpy(&w[10], cell, sizeof(cell));
+  w[16] = 1; // mapc, mapr, maps
+  w[17] = 2;
+  w[18] = 3;
+  const size_t n2 = (size_t) N * N;
+  float mn = n ? maps[0] : 0.f, mx = mn;
+  double sum = 0.0;
+  for (size_t k = 0; k < n2 * n; k++)
+  {
+    mn = std::min(mn, maps[k]);
+    mx = std::max(mx, maps[k]);
+    sum += maps[k];
+  }
+  const float st[3] = {mn, mx, n ? (float) (sum / (double) (n2 * n)) : 0.f};
+  memcpy(&w[19], st, sizeof(st));
+  memcpy(&w[52], "MAP ", 4);
+  w[53] = 0x00004444; // little-endian machine stamp
+  FILE *f = fopen(file.c_str(), "wb");
+  if (!f)
+    fail("Opening file: %s", file.c_str());
+  bool ok = fwrite(w, 4, 256, f) == 256;
+  std::vector<float> t(n2);
+  for (int m = 0; m < n && ok; m++)
+  {
+    const float *img = maps + (size_t) m * n2;
+    for (int i = 0; i < N; i++)
+      for (int j = 0; j < N; j++)
+        t[(size_t) j * N + i] = img[(size_t) i * N + j];
+    ok = fwrite(t.data(), sizeof(float), n2, f) == n2;
+  }
+  if (fclose(f) != 0 || !ok)
+    fail("Writing file: %s", file.c_str());
 }
 
 // --------------------------------------------------------------------------- model

@@ -226,6 +226,19 @@ int bioem_b200_out_of_frame(bioem_b200_handle h, int *perOrient, long long *tota
  * BIOEM_B200_CACHED_PRODUCT=0/1 in the environment overrides the choice for real kernels. */
 int bioem_b200_cached_product(bioem_b200_handle h);
 
+/* The calculated image each record names: maps_out[i][N][N], in the layout of the images given to
+ * upload_particles (RefMap.maps), so that particle - map is the residual.  Reads max_prob_orient, max_prob_conv,
+ * max_prob_cent_x/y (as download() returns them), max_prob_norm and max_prob_mu:
+ *     maps_out[i][x][y] = norm * R0[(x - cent_x) mod N][(y - cent_y) mod N] + mu
+ * where R0 is the convolved projection c2r(P_o K_c) / N^2 (sum R0 = sumC; sum R0^2 is sumsquareC less the part of
+ * the CTF table's non-Hermitian self-conjugate columns that no real image carries), so that render_maps(download())
+ * gives every particle's best-fit map.  Needs model, orientations and CTF table, not
+ * particles or a run.  Synchronous.  Leaves the running state untouched (download(), the angle table,
+ * exact_argmax_info, out_of_frame and stats are what they would have been without the call).  Refuses an
+ * orientation or CTF index out of range, |cent| >= N, n < 0 and null pointers when n > 0 (BIOEM_B200_ERR_INVALID);
+ * missing uploads give BIOEM_B200_ERR_STATE. */
+int bioem_b200_render_maps(bioem_b200_handle h, const bioem_b200_prob_map *records, int n, float *maps_out);
+
 /* ---- inspection entry points (tests): intermediate products of one orientation ---- */
 /* real-space projection (N*N, already scaled by NormDen/tempden) */
 int bioem_b200_debug_projection(bioem_b200_handle h, int iOrient, float *proj_out);
