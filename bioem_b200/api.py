@@ -47,7 +47,8 @@ EXPORTS = [
     "bioem_b200_last_error", "bioem_b200_version", "bioem_b200_device_count",
     "bioem_b200_supported_size", "bioem_b200_create", "bioem_b200_destroy",
     "bioem_b200_upload_model", "bioem_b200_upload_orientations", "bioem_b200_upload_ctf",
-    "bioem_b200_upload_ctf_real", "bioem_b200_upload_particles", "bioem_b200_upload_particles_mrc",
+    "bioem_b200_upload_ctf_real", "bioem_b200_upload_ctf_groups", "bioem_b200_set_particle_groups",
+    "bioem_b200_upload_particles", "bioem_b200_upload_particles_mrc",
     "bioem_b200_upload_particles_fft",
     "bioem_b200_reset",
     "bioem_b200_run", "bioem_b200_synchronize", "bioem_b200_download", "bioem_b200_download_top_angles",
@@ -92,6 +93,8 @@ def lib():
     L.bioem_b200_upload_orientations.argtypes = [vp, fp, C.c_int]
     L.bioem_b200_upload_ctf.argtypes = [vp, fp, fp, C.c_int]
     L.bioem_b200_upload_ctf_real.argtypes = [vp, fp, fp, C.c_int]
+    L.bioem_b200_upload_ctf_groups.argtypes = [vp, fp, fp, fp, C.c_int, C.c_int]
+    L.bioem_b200_set_particle_groups.argtypes = [vp, C.POINTER(C.c_int), C.c_int]
     L.bioem_b200_upload_particles.argtypes = [vp, fp, C.c_int]
     L.bioem_b200_upload_particles_mrc.argtypes = [vp, fp, C.c_int, C.c_int]
     L.bioem_b200_upload_particles_fft.argtypes = [vp, fp, fp, fp, C.c_int]
@@ -181,6 +184,8 @@ class HostInputs:
         sig_a = f32(ctf.get("SIGMA_PRIOR_AMP_CTF", 0.5))
         cen_a = f32(ctf.get("PRIOR_AMP_CTF_CENTER", 0.0))
         self.use_psf = "PSF_PHASE" in ctf
+        self.pixel_size = float(pixel_size)
+        self.elecwavel = float(elecwavel)
         grids = np.zeros(3, dtype=np.float32)
         if not self.use_psf:
             d0, d1, nd = ctf["CTF_DEFOCUS"]
@@ -227,6 +232,36 @@ class HostInputs:
         self.points["density"] = m[:, 4]
         self.NormDen = L.bioem_b200_host_model_prepare(self.points.ctypes.data, len(self.points),
                                                        int(center_model))
+
+    def ctf_groups(self, defocus_um, ctf: dict) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """Per-micrograph CTF tables for upload_ctf_groups: for every defocus value d [micro-m] of defocus_um, the
+        table of ctf's CTF_AMPLITUDE / CTF_B_ENV grids and a CTF_DEFOCUS grid of the same width and count centred on d,
+        with the defocus prior centred on d.  Returns (refCTF [G, C, F, 2], CtfParam [G, C, 4], Priordefcent [G] in
+        phase units)."""
+        if self.use_psf:
+            raise BioemError("ctf_groups: USE_PSF kernels are complex; grouped CTF tables must be real")
+        L = lib()
+        f32 = np.float32
+        d0, d1, nd = ctf["CTF_DEFOCUS"]
+        b0, b1, nb = ctf["CTF_B_ENV"]
+        a0, a1, na = ctf["CTF_AMPLITUDE"]
+        half = f32(0.5) * (f32(d1) - f32(d0))
+        vals = np.asarray(defocus_um, dtype=np.float32).reshape(-1)
+        G = len(vals)
+        ref = np.zeros((G, self.C, self.F, 2), dtype=np.float32)
+        par = np.zeros((G, self.C, 4), dtype=np.float32)
+        cen = np.zeros(G, dtype=np.float32)
+        grids = np.zeros(3, dtype=np.float32)
+        for g, d in enumerate(vals):
+            p0, p1, pc = C.c_float(), C.c_float(), C.c_float(d)
+            L.bioem_b200_host_defocus_to_phase(f32(d - half), f32(d + half), f32(self.elecwavel), C.byref(p0),
+                                               C.byref(p1), C.byref(pc), None)
+            c = L.bioem_b200_host_ctf_table(self.N, f32(self.pixel_size), 0, f32(a0), f32(a1), int(na), p0, p1,
+                                            int(nd), f32(b0), f32(b1), int(nb), _fp(ref[g]), _fp(par[g]), _fp(grids))
+            if c != self.C:
+                raise BioemError(f"ctf_groups: group {g}: {c} kernels, expected {self.C}")
+            cen[g] = pc.value
+        return ref, par, cen
 
     @staticmethod
     def normalise_particles(imgs: np.ndarray) -> np.ndarray:
@@ -287,6 +322,25 @@ class Engine:
         p = np.ascontiguousarray(ctf_param4, dtype=np.float32)
         assert p.shape == (self.C, 4)
         _chk(lib().bioem_b200_upload_ctf_real(self._h, _fp(k), _fp(p), self.C), "upload_ctf_real")
+
+    def upload_ctf_groups(self, refCTF: np.ndarray, ctf_param4: np.ndarray, prior_defocus_center=None):
+        """refCTF [G, C, F, 2] / ctf_param4 [G, C, 4]: G real CTF tables of C rows; prior_defocus_center [G] in phase
+        units (None: the config's centre).  Particle m integrates over its group's rows (set_particle_groups); records
+        name rows of the whole table, g*C + c.  run_capture then returns [O, C, M, nw, nw]."""
+        r = np.ascontiguousarray(refCTF, dtype=np.float32)
+        p = np.ascontiguousarray(ctf_param4, dtype=np.float32)
+        G, Cg = int(r.shape[0]), int(r.shape[1])
+        assert p.shape == (G, Cg, 4)
+        cen = None if prior_defocus_center is None else np.ascontiguousarray(prior_defocus_center, dtype=np.float32)
+        assert cen is None or cen.shape == (G,)
+        _chk(lib().bioem_b200_upload_ctf_groups(self._h, _fp(r), _fp(p), _fp(cen), G, Cg), "upload_ctf_groups")
+        self.C = Cg
+
+    def set_particle_groups(self, group: np.ndarray):
+        """group[M]: every particle's CTF group, in [0, G)."""
+        g = np.ascontiguousarray(group, dtype=np.int32)
+        _chk(lib().bioem_b200_set_particle_groups(self._h, g.ctypes.data_as(C.POINTER(C.c_int)), len(g)),
+             "set_particle_groups")
 
     def upload_particles(self, maps: np.ndarray):
         m = np.ascontiguousarray(maps, dtype=np.float32)

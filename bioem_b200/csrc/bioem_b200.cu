@@ -5,6 +5,7 @@
 #include "render_kernels.cuh"
 
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -103,7 +104,14 @@ struct bioem_b200_context
   int O = 0;
   float4 *d_ctf = nullptr;
   double *d_prior = nullptr;
-  int C = 0;
+  int C = 0; // rows of the CTF table (a grouped table: G x Cg)
+  // Grouped table (upload_ctf_groups): particle m integrates over the Cg rows [group[m]*Cg, group[m]*Cg + Cg) only.
+  // Ungrouped: G = 1, Cg = C and every particle takes every row.
+  int G = 1, Cg = 0;
+  bool grouped = false;
+  bool groups_set = false;                   // set_particle_groups() matches the particles on the handle
+  int group_max = -1;                        // largest group number of that list
+  int *d_group = nullptr, *d_perm = nullptr; // [M] group of every particle; particles ordered by group
   // cached-product mode of the fused kernel (LikParams::zmode): possible when every CTF kernel is real (CTFs given
   // in Fourier space), chosen in ensure_batch
   bool ctf_is_real = false, zmode = false;
@@ -425,6 +433,27 @@ static cudaError_t do_fft2d(int N, const float *imgs, const double *tempden, int
   }
   return cudaErrorInvalidValue;
 }
+template <int N>
+static cudaError_t launch_sums(const float4 *proj, const float4 *ctf, const double *prior, ConvParam *cpar, int GC, int OBcur,
+                               float Nt, cudaStream_t s)
+{
+  dim3 g((GC + SUMS_CB - 1) / SUMS_CB, (OBcur + SUMS_OB - 1) / SUMS_OB);
+  ctf_sums_kernel<N><<<g, NT, 0, s>>>(proj, ctf, prior, cpar, GC, OBcur, Nt);
+  return cudaGetLastError();
+}
+static cudaError_t do_sums(int N, const float4 *proj, const float4 *ctf, const double *prior, ConvParam *cpar, int GC,
+                           int OBcur, float Nt, cudaStream_t s)
+{
+  switch (N)
+  {
+#define X(n)                                                                                              \
+  case n:                                                                                                 \
+    return launch_sums<n>(proj, ctf, prior, cpar, GC, OBcur, Nt, s);
+    BIOEM_SIZES(X)
+#undef X
+  }
+  return cudaErrorInvalidValue;
+}
 static cudaError_t do_conv(int N, const float4 *proj, const float4 *ctf, const double *prior, float4 *conv, ConvParam *cpar,
                            int C, int OBcur, float Nt, cudaStream_t s, const int4 *sel = nullptr, int nsel = 0)
 {
@@ -518,19 +547,24 @@ static size_t smem_for(int N, int maxD, int nwp)
   return 0;
 }
 
-// Gaussian priors on the CTF parameters (bioem_algorithm.h:49-67), per kernel, in double
-static int set_ctf_priors(bioem_b200_context *h, const float *CtfParam4, int C)
+// Gaussian priors on the CTF parameters (bioem_algorithm.h:49-67), per kernel, in double.  A grouped table (G > 1 or
+// cent != nullptr) has G groups of C / G rows, and group r's defocus prior is centred on cent[r] (nullptr: the config's
+// centre for all).
+static int set_ctf_priors(bioem_b200_context *h, const float *CtfParam4, int C, int G = 1, const float *cent = nullptr,
+                          bool grouped = false)
 {
   std::vector<double> prior(C);
   const bioem_b200_config &p = h->cfg;
+  const int Cg = C / G;
   for (int c = 0; c < C; c++)
   {
     const float amp = CtfParam4[4 * c], pha = CtfParam4[4 * c + 1], env = CtfParam4[4 * c + 2];
+    const float dcen = cent ? cent[c / Cg] : p.Priordefcent;
     double pr;
     if (!p.tousepsf)
     {
       pr = env * env / 2. / p.sigmaPriorbctf / p.sigmaPriorbctf -
-           (pha - p.Priordefcent) * (pha - p.Priordefcent) / 2. / p.sigmaPriordefo / p.sigmaPriordefo -
+           (pha - dcen) * (pha - dcen) / 2. / p.sigmaPriordefo / p.sigmaPriordefo -
            (amp - p.Priorampcent) * (amp - p.Priorampcent) / 2. / p.sigmaPrioramp / p.sigmaPrioramp;
     }
     else
@@ -549,9 +583,15 @@ static int set_ctf_priors(bioem_b200_context *h, const float *CtfParam4, int C)
   h->state_ready = false;
   (void) Cold;
   free_batch(h); // (also when C is unchanged: a real / complex table decides the mode of the fused kernel)
+  // an ungrouped table drops the particle groups; a grouped one keeps them while they name groups it has
+  h->groups_set = grouped && h->groups_set && h->group_max < G;
+  h->grouped = false;
   RC(dev_realloc(h, h->d_prior, (size_t) C));
   CU(cudaMemcpyAsync(h->d_prior, prior.data(), sizeof(double) * C, cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));
+  h->G = G;
+  h->Cg = Cg;
+  h->grouped = grouped;
   h->C = C;
   return BIOEM_B200_OK;
 }
@@ -718,6 +758,8 @@ int bioem_b200_destroy(bioem_b200_handle h)
   dfree(h, h->d_ctf);
   dfree(h, h->d_kreal);
   dfree(h, h->d_prior);
+  dfree(h, h->d_group);
+  dfree(h, h->d_perm);
   dfree(h, h->d_refs);
   dfree(h, h->d_sumRef);
   dfree(h, h->d_sumsqRef);
@@ -787,10 +829,10 @@ int bioem_b200_upload_orientations(bioem_b200_handle h, const float *angles4, in
   return BIOEM_B200_OK;
 }
 
-int bioem_b200_upload_ctf(bioem_b200_handle h, const float *refCTF, const float *CtfParam4, int C)
+// upload_ctf and upload_ctf_groups (G groups of C / G rows)
+static int upload_ctf_table(bioem_b200_context *h, const float *refCTF, const float *CtfParam4, int C, int G,
+                            const float *cent, bool grouped)
 {
-  if (!h || !refCTF || !CtfParam4 || C <= 0)
-    return fail(BIOEM_B200_ERR_INVALID, "upload_ctf: bad argument");
   CU(cudaSetDevice(h->device));
   const int N = h->N;
   const size_t stdsz = (size_t) N * (N / 2 + 1);
@@ -823,7 +865,35 @@ int bioem_b200_upload_ctf(bioem_b200_handle h, const float *refCTF, const float 
   }
   CU(cudaStreamSynchronize(h->stream));
   h->C = Cold;
-  return set_ctf_priors(h, CtfParam4, C);
+  return set_ctf_priors(h, CtfParam4, C, G, cent, grouped);
+}
+
+int bioem_b200_upload_ctf(bioem_b200_handle h, const float *refCTF, const float *CtfParam4, int C)
+{
+  if (!h || !refCTF || !CtfParam4 || C <= 0)
+    return fail(BIOEM_B200_ERR_INVALID, "upload_ctf: bad argument");
+  return upload_ctf_table(h, refCTF, CtfParam4, C, 1, nullptr, false);
+}
+
+int bioem_b200_upload_ctf_groups(bioem_b200_handle h, const float *refCTF, const float *CtfParam4, const float *Priordefcent,
+                                 int G, int C)
+{
+  if (!h || !refCTF || !CtfParam4)
+    return fail(BIOEM_B200_ERR_INVALID, "upload_ctf_groups: null handle or table");
+  if (G < 1 || C < 1 || (long long) G * C > INT_MAX / 2)
+    return fail(BIOEM_B200_ERR_INVALID, "upload_ctf_groups: G = " + std::to_string(G) + ", C = " + std::to_string(C) +
+                                            ": need G >= 1 and C >= 1");
+  if (h->generic)
+    return fail(BIOEM_B200_ERR_INVALID, "upload_ctf_groups: NUMBER_PIXELS " + std::to_string(h->N) +
+                                            " runs on the direct-DFT path, which takes no grouped CTF table");
+  if (h->cfg.tousepsf)
+    return fail(BIOEM_B200_ERR_INVALID, "upload_ctf_groups: USE_PSF kernels are complex; grouped tables must be real");
+  const size_t n = (size_t) h->N * (h->N / 2 + 1) * G * C;
+  for (size_t i = 0; i < n; i++)
+    if (refCTF[2 * i + 1] != 0.f)
+      return fail(BIOEM_B200_ERR_INVALID, "upload_ctf_groups: row " + std::to_string(i / (n / ((size_t) G * C))) +
+                                              " has a non-zero imaginary part; grouped tables must be real");
+  return upload_ctf_table(h, refCTF, CtfParam4, G * C, G, Priordefcent, true);
 }
 
 int bioem_b200_upload_ctf_real(bioem_b200_handle h, const float *kernels, const float *CtfParam4, int C)
@@ -855,6 +925,7 @@ int bioem_b200_upload_ctf_real(bioem_b200_handle h, const float *kernels, const 
 static int begin_particles(bioem_b200_context *h, int M, size_t *cap)
 {
   h->state_ready = false;
+  h->groups_set = false; // a new stack needs its own group list
   const bool same = (size_t) M == *cap && h->d_refs && h->d_sumRef && h->d_sumsqRef && h->d_state && h->d_out;
   h->M = 0;
   if (!same)
@@ -962,10 +1033,50 @@ int bioem_b200_upload_particles_fft(bioem_b200_handle h, const float *fft, const
   return BIOEM_B200_OK;
 }
 
+int bioem_b200_set_particle_groups(bioem_b200_handle h, const int *group, int M)
+{
+  if (!h || !group)
+    return fail(BIOEM_B200_ERR_INVALID, "set_particle_groups: null handle or list");
+  if (h->M <= 0 || !h->grouped || h->C <= 0)
+    return fail(BIOEM_B200_ERR_STATE, "set_particle_groups: upload the particles and a grouped CTF table first");
+  if (M != h->M)
+    return fail(BIOEM_B200_ERR_INVALID, "set_particle_groups: " + std::to_string(M) + " entries for " + std::to_string(h->M) +
+                                            " particles");
+  int gmax = -1;
+  for (int m = 0; m < M; m++)
+  {
+    if (group[m] < 0 || group[m] >= h->G)
+      return fail(BIOEM_B200_ERR_INVALID, "set_particle_groups: particle " + std::to_string(m) + ": group " +
+                                              std::to_string(group[m]) + " out of range [0, " + std::to_string(h->G) + ")");
+    gmax = std::max(gmax, group[m]);
+  }
+  CU(cudaSetDevice(h->device));
+  h->state_ready = false;
+  h->groups_set = false;
+  // CTAs take the particles group by group: the resident ones share one or two groups' tables in L2
+  std::vector<int> perm((size_t) M);
+  for (int m = 0; m < M; m++)
+    perm[m] = m;
+  std::stable_sort(perm.begin(), perm.end(), [&](int a, int b) { return group[a] < group[b]; });
+  RC(dev_realloc(h, h->d_group, (size_t) M));
+  RC(dev_realloc(h, h->d_perm, (size_t) M));
+  CU(cudaMemcpyAsync(h->d_group, group, sizeof(int) * M, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(h->d_perm, perm.data(), sizeof(int) * M, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  h->group_max = gmax;
+  h->groups_set = true;
+  return BIOEM_B200_OK;
+}
+
 static int ensure_batch(bioem_b200_context *h)
 {
   if (h->OB > 0)
     return BIOEM_B200_OK;
+  // a grouped table runs in cached-product mode only (its kernels are real and the fused kernel's grouped variant is a
+  // cached-product one): the environment cannot switch that mode off for it
+  if (h->grouped && getenv("BIOEM_B200_CACHED_PRODUCT") && atoi(getenv("BIOEM_B200_CACHED_PRODUCT")) == 0)
+    return fail(BIOEM_B200_ERR_INVALID, "run: a grouped CTF table needs the cached-product mode; "
+                                        "BIOEM_B200_CACHED_PRODUCT=0 is not supported with it");
   const int N = h->N;
   const size_t mapbytes = h->map4 * sizeof(float4);
   // Orientations per batch: the conv spectra of a batch live in HBM (1 GB budget); what has to stay
@@ -985,6 +1096,11 @@ static int ensure_batch(bioem_b200_context *h)
   if (env_pos("BIOEM_B200_CONV_MB"))
     budget = (size_t) env_pos("BIOEM_B200_CONV_MB") << 20;
   long ob = (long) (budget / (mapbytes * (size_t) h->C));
+  // a grouped table keeps no conv spectra: per orientation a batch holds its projection (image, r2c scratch, packed
+  // spectrum), its G x C conv parameters and at most one partial per particle
+  if (h->grouped)
+    ob = (long) (budget / ((size_t) N * N * sizeof(float) + (size_t) N * (N / 2 + 1) * sizeof(float2) + mapbytes +
+                           (size_t) h->C * sizeof(ConvParam) + (size_t) h->M * sizeof(Running)));
   ob = std::max<long>(1, std::min<long>(ob, h->O));
   if (env_pos("BIOEM_B200_OB"))
     ob = std::max<long>(1, std::min<long>(env_pos("BIOEM_B200_OB"), h->O));
@@ -1000,7 +1116,7 @@ static int ensure_batch(bioem_b200_context *h)
   // cannot be run ahead) over >= 64 likelihoods, keep >= 4 waves (cfg2: 1 -> 2 orientations, +0.5 %)
   // (above N = 224, one CTA per SM, more than one orientation per CTA at 32 CTFs costs 3-5 %)
   const int per_cta = h->N <= 224 ? 64 : 16;
-  int og = std::max(1, (per_cta + h->C - 1) / h->C);
+  int og = std::max(1, (per_cta + h->Cg - 1) / h->Cg);
   const long long cta_slots = h->N <= 128 ? 592 : h->N <= 224 ? 296 : 148; // resident CTAs of the fused kernel per GPU
   while (og > 1 && (long long) h->M * ((h->OB + og - 1) / og) < 4LL * cta_slots)
     og--;
@@ -1040,6 +1156,8 @@ static int ensure_batch(bioem_b200_context *h)
   bool zmode = h->ctf_is_real && h->d_kreal && h->C >= 4;
   if (const char *v = getenv("BIOEM_B200_CACHED_PRODUCT"))
     zmode = h->ctf_is_real && h->d_kreal && atoi(v) != 0;
+  if (h->grouped)
+    zmode = true;
   if (h->generic)
   {
     zmode = false;
@@ -1058,7 +1176,8 @@ static int ensure_batch(bioem_b200_context *h)
     h->nslots = nslots;
   }
   // (in that mode only the inspection entry point debug_convolved wants convolved spectra: one orientation's worth)
-  RC(dev_realloc(h, h->d_conv, h->map4 * (size_t) (zmode ? 1 : OB) * h->C));
+  // (a grouped table: one conv spectrum, debug_convolved forms the one it is asked for)
+  RC(dev_realloc(h, h->d_conv, h->map4 * (size_t) (zmode ? 1 : OB) * (h->grouped ? 1 : h->C)));
   RC(dev_realloc(h, h->d_cpar, (size_t) OB * h->C));
   h->partials_cap = (size_t) h->M * ((OB + h->OG - 1) / h->OG);
   RC(dev_realloc(h, h->d_partials, h->partials_cap));
@@ -1133,7 +1252,10 @@ static int run_front(bioem_b200_context *h, int o0, int OBcur, const float4 *ang
   float4 *conv = (h->zmode && !want_conv) ? nullptr : h->d_conv; // (want_conv in cached-product mode: OBcur == 1)
   if (want_conv && conv_dst)
     conv = conv_dst;
-  CU(do_conv(N, h->d_projfft, h->d_ctf, h->d_prior, conv, h->d_cpar, h->C, OBcur, h->cfg.Ntotpi, h->stream, sel, nsel));
+  if (h->grouped && !conv && !sel)
+    CU(do_sums(N, h->d_projfft, h->d_ctf, h->d_prior, h->d_cpar, h->C, OBcur, h->cfg.Ntotpi, h->stream));
+  else
+    CU(do_conv(N, h->d_projfft, h->d_ctf, h->d_prior, conv, h->d_cpar, h->C, OBcur, h->cfg.Ntotpi, h->stream, sel, nsel));
   h->launches += 4;
   return BIOEM_B200_OK;
 }
@@ -1160,7 +1282,10 @@ static void fill_lik_params(bioem_b200_context *h, LikParams &lp, int o0, int OB
   lp.kr4 = (int) h->kr4;
   lp.zmode = h->zmode ? 1 : 0;
   lp.M = h->M;
-  lp.C = h->C;
+  lp.C = h->Cg; // rows per particle; the grouped variant's particles take theirs out of lp.GC
+  lp.GC = h->C;
+  lp.group = h->grouped ? h->d_group : nullptr;
+  lp.perm = h->grouped ? h->d_perm : nullptr;
   lp.OBcur = OBcur;
   lp.OG = h->OG;
   lp.o_base = o0;
@@ -1206,6 +1331,8 @@ static int run_range(bioem_b200_context *h, int oBegin, int oEnd, float *capture
     return fail(BIOEM_B200_ERR_INVALID, "run: null handle");
   if (h->A <= 0 || h->O <= 0 || h->C <= 0 || h->M <= 0)
     return fail(BIOEM_B200_ERR_STATE, "run: model, orientations, CTF table and particles must be uploaded first");
+  if (h->grouped && !h->groups_set)
+    return fail(BIOEM_B200_ERR_STATE, "run: a grouped CTF table needs the particles' groups (set_particle_groups)");
   if (oBegin < 0 || oEnd > h->O || oBegin > oEnd)
     return fail(BIOEM_B200_ERR_INVALID, "run: orientation range out of bounds");
   CU(cudaSetDevice(h->device));
@@ -1226,7 +1353,7 @@ static int run_range(bioem_b200_context *h, int oBegin, int oEnd, float *capture
       return rc;
     // capture: the batch's windows land in a temp (fused kernel) or in d_values (direct-DFT path), prefilled with
     // 0xFF bytes -- a NaN -- so that an entry the kernel does not write shows up
-    const size_t ncap = capture ? (size_t) OBcur * h->C * h->M * h->nw * h->nw : 0;
+    const size_t ncap = capture ? (size_t) OBcur * h->Cg * h->M * h->nw * h->nw : 0;
     DevTmp t_cap(h);
     float *d_cap = nullptr;
     if (capture)
@@ -1272,7 +1399,7 @@ static int run_range(bioem_b200_context *h, int oBegin, int oEnd, float *capture
     h->lik_launches += 1;
     if (capture)
     {
-      CU(cudaMemcpyAsync(capture + (size_t) (o0 - oBegin) * h->C * h->M * h->nw * h->nw, d_cap, sizeof(float) * ncap,
+      CU(cudaMemcpyAsync(capture + (size_t) (o0 - oBegin) * h->Cg * h->M * h->nw * h->nw, d_cap, sizeof(float) * ncap,
                          cudaMemcpyDeviceToHost, h->stream));
       CU(cudaStreamSynchronize(h->stream));
     }
@@ -1281,7 +1408,7 @@ static int run_range(bioem_b200_context *h, int oBegin, int oEnd, float *capture
     merge_partials_kernel<<<(h->M + 127) / 128, 128, 0, h->stream>>>(h->d_partials, NG, h->M, h->d_state);
     CU(cudaGetLastError());
     h->launches += 2;
-    h->likelihoods += (long long) OBcur * h->C * h->M;
+    h->likelihoods += (long long) OBcur * h->Cg * h->M;
     h->argmax_exact = false;
   }
   return BIOEM_B200_OK;
@@ -1358,6 +1485,7 @@ static int refine_argmax(bioem_b200_context *h)
     fill_lik_params(h, lp, 0, (int) items.size()); // one "orientation" of one CTF per item
     lp.C = 1;
     lp.OG = 1;
+    lp.group = lp.perm = nullptr; // (the items name rows of the whole table)
     lp.pairs = t_items.as<int4>();
     lp.partials = t_part.as<Running>();
     lp.angles = nullptr;
@@ -1994,7 +2122,18 @@ int bioem_b200_debug_convolved(bioem_b200_handle h, int o, int c, float *conv_ou
   int rc = ensure_batch(h);
   if (rc)
     return rc;
-  rc = run_front(h, o, 1, nullptr, nullptr, 0, true);
+  // (a grouped table: only row c is convolved, through the selection path, into slot 0)
+  DevTmp t_sel(h);
+  if (h->grouped)
+  {
+    const int4 one = make_int4(0, 0, c, 0);
+    RC(t_sel.alloc(sizeof(int4)));
+    CU(cudaMemcpyAsync(t_sel.p, &one, sizeof(int4), cudaMemcpyHostToDevice, h->stream));
+    rc = run_front(h, o, 1, nullptr, t_sel.as<int4>(), 1, true);
+    c = 0;
+  }
+  else
+    rc = run_front(h, o, 1, nullptr, nullptr, 0, true);
   if (rc)
     return rc;
   const size_t stdsz = (size_t) h->N * (h->N / 2 + 1);
@@ -2054,6 +2193,8 @@ int bioem_b200_debug_correlation(bioem_b200_handle h, int o, int c, int m, float
   lp.dbg_values = d_dbg;
   lp.M = 1;
   lp.OG = 1;
+  lp.C = h->C; // every row of the table (a grouped one too)
+  lp.group = lp.perm = nullptr;
   CU(do_lik(h->N, lp, 1, h->cfg.maxDisplaceCenter, h->stream));
   CU(cudaMemcpyAsync(values, d_dbg + (size_t) c * nv, sizeof(float) * nv, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));

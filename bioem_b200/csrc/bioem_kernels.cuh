@@ -710,6 +710,101 @@ __global__ void __launch_bounds__(NT) ctf_conv_kernel(const float4 *__restrict__
   }
 }
 
+// Stage 2 of a grouped CTF table (cached-product mode, G x C rows): only sumC, sumsquareC and the B-term, for every
+// (orientation, row) pair of the batch.  ctf_conv_kernel makes one pass over a projection and a table row per pair;
+// here a CTA takes SUMS_CB rows x SUMS_OB orientations and loads every float4 of them once for all SUMS_CB x SUMS_OB
+// pairs (the G x C rows do not fit L2; the table is read OBcur / SUMS_OB times per batch instead of OBcur times).
+// Each pair's sum runs in exactly the order of ctf_conv_kernel (same per-thread stride, same tree), so cpar is
+// bit-identical to what ctf_conv_kernel writes for the same row.  Output slot ob*GC + row.
+constexpr int SUMS_CB = 4, SUMS_OB = 8;
+template <int N>
+__global__ void __launch_bounds__(NT) ctf_sums_kernel(const float4 *__restrict__ proj, const float4 *__restrict__ ctf,
+                                                      const double *__restrict__ prior, ConvParam *__restrict__ cpar,
+                                                      int GC, int OBcur, float Ntotpi)
+{
+  using L = Lay<N>;
+  const int tid = threadIdx.x;
+  const int c0 = blockIdx.x * SUMS_CB, o0 = blockIdx.y * SUMS_OB;
+  const float4 *K[SUMS_CB];
+  const float4 *P[SUMS_OB];
+#pragma unroll
+  for (int j = 0; j < SUMS_CB; j++)
+    K[j] = ctf + (size_t) min(c0 + j, GC - 1) * L::MAP4; // (past the end: a valid row, never written out)
+#pragma unroll
+  for (int b = 0; b < SUMS_OB; b++)
+    P[b] = proj + (size_t) min(o0 + b, OBcur - 1) * L::MAP4;
+  __shared__ float red[SUMS_OB * SUMS_CB][NT];
+  __shared__ float s_sumC[SUMS_OB * SUMS_CB]; // kx = 0, ky = 0 of every pair
+  float acc[SUMS_OB][SUMS_CB];
+#pragma unroll
+  for (int b = 0; b < SUMS_OB; b++)
+#pragma unroll
+    for (int j = 0; j < SUMS_CB; j++)
+      acc[b][j] = 0.f;
+  for (int i = tid; i < L::MAP4; i += NT)
+  {
+    float w = 2.f;
+    const bool tail = i >= L::MAIN4;
+    int n1p, n2, ky;
+    L::decode(i, n1p, n2, ky);
+    if (tail || ky == 0)
+      w = 1.f;
+    float4 k[SUMS_CB];
+#pragma unroll
+    for (int j = 0; j < SUMS_CB; j++)
+      k[j] = K[j][i];
+#pragma unroll
+    for (int b = 0; b < SUMS_OB; b++)
+    {
+      const float4 a = P[b][i];
+#pragma unroll
+      for (int j = 0; j < SUMS_CB; j++)
+      {
+        float4 v;
+        v.x = a.x * k[j].x + a.y * k[j].y;
+        v.y = a.y * k[j].x - a.x * k[j].y;
+        v.z = a.z * k[j].z + a.w * k[j].w;
+        v.w = a.w * k[j].z - a.z * k[j].w;
+        acc[b][j] += w * (v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w);
+        if (i == 0)
+          s_sumC[b * SUMS_CB + j] = v.x;
+      }
+    }
+  }
+#pragma unroll
+  for (int b = 0; b < SUMS_OB; b++)
+#pragma unroll
+    for (int j = 0; j < SUMS_CB; j++)
+      red[b * SUMS_CB + j][tid] = acc[b][j];
+  __syncthreads();
+  for (int s = NT / 2; s > 0; s >>= 1)
+  {
+    if (tid < s)
+#pragma unroll
+      for (int q = 0; q < SUMS_OB * SUMS_CB; q++)
+        red[q][tid] += red[q][tid + s];
+    __syncthreads();
+  }
+  if (tid == 0)
+#pragma unroll
+    for (int b = 0; b < SUMS_OB; b++)
+#pragma unroll
+      for (int j = 0; j < SUMS_CB; j++)
+      {
+        const int c = c0 + j, ob = o0 + b;
+        if (c >= GC || ob >= OBcur)
+          continue;
+        const float ssC = __fdiv_rn(red[b * SUMS_CB + j][0], (float) (N * N));
+        const float sC = s_sumC[b * SUMS_CB + j];
+        ConvParam cp;
+        cp.sumC = sC;
+        cp.sumsqC = ssC;
+        const float fl = __fsub_rn(__fmul_rn(ssC, Ntotpi), __fmul_rn(sC, sC));
+        cp.Bterm = ((double) Ntotpi * 0.5 - 2.0) * log((double) __fsub_rn(Ntotpi, 2.f) * (double) fl) - prior[c];
+        cpar[(size_t) ob * GC + c] = cp;
+      }
+}
+
 struct LikParams
 {
   const float4 *convs; // [OBcur*C][MAP4]
@@ -742,6 +837,12 @@ struct LikParams
   float invNN;
   float ex2coef; // (3 - Nt)/2 * log2(e): sum of exp over the window runs in base 2
   double acoef_d;
+  // grouped CTF table (likelihood_kernel<N, W, true, true>, chosen by group != nullptr; cached-product mode only):
+  // kreal / cpar hold GC = G x C rows, particle m integrates over the C rows [group[m]*C, group[m]*C + C) of them;
+  // CTA b takes particle perm[b % M] (particles ordered by group, so the resident CTAs share few groups' tables)
+  const int *group; // [M]
+  const int *perm;  // [M]
+  int GC;
 };
 
 // Real CTF table of the cached-product mode, per CTF, in the order the column pass consumes it: lane
@@ -1005,7 +1106,7 @@ struct BookState
 // -> rows) and one split-phase mbarrier (rows -> next columns: arrive, run the first radix pass
 // of the next likelihood's first chunk, wait); no correlation map ever leaves the SM.
 // ===========================================================================
-template <int N, int W, bool ZM>
+template <int N, int W, bool ZM, bool GR = false>
 __global__ void __launch_bounds__(LikSmem<N>::LNT) __maxnreg__(LikSmem<N>::MAXREG) likelihood_kernel(LikParams p)
 {
   using KL = KLay<N>;
@@ -1064,7 +1165,10 @@ __global__ void __launch_bounds__(LikSmem<N>::LNT) __maxnreg__(LikSmem<N>::MAXRE
   if constexpr ((RV & 16) != 0)
     asm volatile("" : "+r"(warp));
   float2 *E = Eall + (size_t) warp * SM::EW;
-  const int m = p.pairs ? p.pairs[blockIdx.x].x : blockIdx.x % p.M;
+  static_assert(ZM || !GR, "grouped CTF tables are real: cached-product mode only");
+  const int m = GR ? p.perm[blockIdx.x % p.M] : (p.pairs ? p.pairs[blockIdx.x].x : blockIdx.x % p.M);
+  // (grouped table: first row of this particle's group; the work-list path indexes rows directly and is never grouped)
+  const int cb = GR ? p.group[m] * p.C : 0;
   const int g = p.pairs ? blockIdx.x : blockIdx.x / p.M;
   const int o_lo = g * p.OG;
   const int o_hi = min(p.OBcur, o_lo + p.OG);
@@ -1241,8 +1345,8 @@ __global__ void __launch_bounds__(LikSmem<N>::LNT) __maxnreg__(LikSmem<N>::MAXRE
         s_bk.Total = s_bk.Total * exp(s_bk.Const - (double) lpfmax) + e;
         s_bk.Const = (double) lpfmax;
         s_bk.lpf = lpfmax;
-        s_bk.o = p.o_base + oc / p.C;
-        s_bk.c = oc % p.C;
+        s_bk.o = p.o_base + oc / (GR ? p.GC : p.C);
+        s_bk.c = oc % (GR ? p.GC : p.C); // (grouped: the row of the whole table)
         s_bk.lin = 0; // displacement index and correlation value: filled in by the exact pass
         s_bk.v = 0.f;
         s_bk.sC = cpl.sumC;
@@ -1546,17 +1650,18 @@ __global__ void __launch_bounds__(LikSmem<N>::LNT) __maxnreg__(LikSmem<N>::MAXRE
     for (int c = 0; c < p.C; c++)
     {
       const int oc = ol * p.C + c;
+      const int orow = GR ? ol * p.GC + cb + c : oc; // row of cpar (grouped: [OBcur][GC])
       // (cached-product mode: the real table of CTF c, or of the work item's CTF)
-      int koff = ZM ? (p.pairs ? p.pairs[blockIdx.x].z : c) * p.kr4 : 0;
+      int koff = ZM ? (p.pairs ? p.pairs[blockIdx.x].z : cb + c) * p.kr4 : 0;
       if constexpr (ZM && (BIOEM_ZV & 8))
         asm volatile("" : "+r"(koff));
       const float4 *conv = ZM ? p.kreal + koff : p.convs + (size_t) oc * L::MAP4;
       if (tid == 0)
-        s_poc[slot] = oc;
+        s_poc[slot] = orow;
       float sumC, sumsqC;
       if constexpr (!LATE_SUMS)
       {
-        const ConvParam cp = p.cpar[oc];
+        const ConvParam cp = p.cpar[orow];
         sumC = cp.sumC, sumsqC = cp.sumsqC;
       }
 
@@ -1574,7 +1679,7 @@ __global__ void __launch_bounds__(LikSmem<N>::LNT) __maxnreg__(LikSmem<N>::MAXRE
       // firstele = Nt*(ssR*ssC - v*v) + 2*sR*sC*v - ssR*sC*sC - sR*sR*ssC   (FP32, source order)
       // (the loads are issued here; their values are first needed in the epilogue of the first row task)
       if constexpr (LATE_SUMS)
-        sumC = __ldg(&p.cpar[oc].sumC), sumsqC = __ldg(&p.cpar[oc].sumsqC);
+        sumC = __ldg(&p.cpar[orow].sumC), sumsqC = __ldg(&p.cpar[orow].sumsqC);
       const float sR = LATE_SUMS ? s_sr[0] : sR0, ssR = LATE_SUMS ? s_sr[1] : ssR0;
       const float f_a = __fmul_rn(ssR, sumsqC);
       const float f_b = __fmul_rn(__fmul_rn(2.f, sR), sumC);
@@ -1763,7 +1868,7 @@ __global__ void __launch_bounds__(LikSmem<N>::LNT) __maxnreg__(LikSmem<N>::MAXRE
           const bool last = c == p.C - 1;
           if (last)
             zpass(ol + 1);
-          col1(ch0, last ? p.kreal : conv + p.kr4, false);
+          col1(ch0, last ? p.kreal + (size_t) cb * p.kr4 : conv + p.kr4, false);
         }
         else
           col1(ch0, conv + L::MAP4, oc + 2 < o_hi * p.C); // the next conv spectrum of the batch follows this one

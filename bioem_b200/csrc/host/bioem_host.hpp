@@ -23,6 +23,7 @@ struct Options // reference bioem.cpp:193-224
   bool printCoordRead = false;
   int gpus = 0; // extension: number of GPUs of this box to use (0 = all visible)
   std::string bestmapsfile; // extension: --WriteBestMaps, every particle's best-fit calculated map (MRC stack)
+  std::string defocusfile;  // extension: --DefocusPerParticle, one defocus [micro-m] per particle (CTF groups)
 };
 
 struct Params // reference bioem_param after readParameters + CalculateGridsParam + CalculateRefCTF
@@ -39,6 +40,7 @@ struct Params // reference bioem_param after readParameters + CalculateGridsPara
   float sigmaPriorbctf = 100.f, sigmaPriordefo = 2.0f, Priordefcent = 3.0f, sigmaPrioramp = 0.5f, Priorampcent = 0.f;
   int angleGridPointsAlpha = 0, angleGridPointsBeta = 0, GridPointsQuatern = -1;
   float startAmp = 0, endAmp = 0, startPhase = 0, endPhase = 0, startEnv = 0, endEnv = 0;
+  float startDef = 0, endDef = 0; // CTF_DEFOCUS [micro-m]
   int nAmp = 0, nPhase = 0, nEnv = 0;
   // derived
   std::vector<float> angles;   // nOrient x {pos[3], quat4}
@@ -46,8 +48,11 @@ struct Params // reference bioem_param after readParameters + CalculateGridsPara
   float voluang = 0.f;
   std::vector<float> psfKernels; // USE_PSF: nCtf x N x N real-space kernels (refCTF stays empty)
   std::vector<float> refCTF;   // nCtf x N x (N/2+1) x 2
-  std::vector<float> CtfParam; // nCtf x 4 {amp, phase, env, -}
-  int nCtf = 0;
+  std::vector<float> CtfParam; // nCtf x 4 {amp, phase, env, -} (CTF groups: nGroups x nCtf rows, group-major)
+  int nCtf = 0;                // CTF rows every particle integrates over
+  int nGroups = 0;             // --DefocusPerParticle: number of CTF groups (0 = one table for all particles)
+  std::vector<int> group;      // nMaps: CTF group of every particle
+  std::vector<float> groupDefcent; // nGroups: defocus-prior centre of every group [phase]
   float volu = 0.f;
   int nOrient() const { return (int) (angles.size() / 4); }
 };
@@ -56,6 +61,9 @@ void parse_options(int argc, char **argv, Options &o);
 void read_parameters(const std::string &file, Params &p);                  // param.cpp:64-627
 void make_orientations(const std::string &orientfile, Params &p);          // param.cpp:988-1334
 void make_ctf_table(Params &p);                                            // param.cpp:1336-1620 via the C ABI
+// --DefocusPerParticle: one CTF table per distinct defocus of the file (groups in order of first appearance), each with
+// CTF_DEFOCUS's width and count centred on that value and PRIOR_DEFOCUS_CENTER = that value; replaces the table
+void make_ctf_groups(const std::string &file, int nMaps, Params &p);
 void read_model(const Options &o, const Params &p, std::vector<bioem_b200_model_point> &pts, float &NormDen);
 // maps: nMaps x N x N.  For MRC stacks (rawMRC = true) the images are left exactly as they lie in the
 // file; the library transposes / normalises them on the device (bioem_b200_upload_particles_mrc).

@@ -3,7 +3,7 @@
 //   bioEM_b200 --Modelfile m --Particlesfile p --Inputfile i [--ReadOrientation o] [--ReadPDB]
 //              [--ReadModelMRC] [--ReadMRC] [--ReadMultipleMRC] [--DumpMaps] [--LoadMapDump]
 //              [--DumpModel] [--LoadModelDump] [--PrintCOORDREAD] [--OutputFile f] [--Gpus n]
-//              [--WriteBestMaps f]
+//              [--WriteBestMaps f] [--DefocusPerParticle f]
 //
 // Flow = the reference's main.cpp:34-140 / bioem::configure / bioem::run with the main loop
 // (bioem.cpp:763-891) replaced by bioem_b200_run on every GPU of the box: the orientation grid is
@@ -188,6 +188,12 @@ int main(int argc, char **argv)
   read_model(opt, par, pts, NormDen);
   make_orientations(opt.orientfile, par);
   make_ctf_table(par);
+  if (!opt.defocusfile.empty())
+  {
+    if (getenv("BIOEM_DEBUG_BREAK") || getenv("BIOEM_B200_DUMP_INPUTS"))
+      fail("--DefocusPerParticle: BIOEM_DEBUG_BREAK / BIOEM_B200_DUMP_INPUTS take one CTF table");
+    make_ctf_groups(opt.defocusfile, nMaps, par);
+  }
 
   int O = par.nOrient(), C = par.nCtf;
   if (getenv("BIOEM_DEBUG_BREAK")) // the reference's debugging knob (bioem.cpp:518-525)
@@ -292,12 +298,15 @@ int main(int argc, char **argv)
     chk(bioem_b200_create(&cfg, g % nphys, &h), "create") &&
         chk(bioem_b200_upload_model(h, pts.data(), (int) pts.size(), NormDen), "upload_model") &&
         chk(bioem_b200_upload_orientations(h, par.angles.data(), O), "upload_orientations") &&
-        chk(par.usepsf ? bioem_b200_upload_ctf_real(h, par.psfKernels.data(), par.CtfParam.data(), C)
-                       : bioem_b200_upload_ctf(h, par.refCTF.data(), par.CtfParam.data(), C),
+        chk(par.nGroups ? bioem_b200_upload_ctf_groups(h, par.refCTF.data(), par.CtfParam.data(), par.groupDefcent.data(),
+                                                       par.nGroups, C)
+            : par.usepsf ? bioem_b200_upload_ctf_real(h, par.psfKernels.data(), par.CtfParam.data(), C)
+                         : bioem_b200_upload_ctf(h, par.refCTF.data(), par.CtfParam.data(), C),
             "upload_ctf") &&
         chk(rawMRC ? bioem_b200_upload_particles_mrc(h, maps.data(), nMaps, par.notnormmap ? 0 : 1)
                    : bioem_b200_upload_particles(h, maps.data(), nMaps),
             "upload_particles") &&
+        (!par.nGroups || chk(bioem_b200_set_particle_groups(h, par.group.data(), nMaps), "set_particle_groups")) &&
         chk(bioem_b200_reset(h), "reset") && chk(bioem_b200_run(h, o0, o1), "run") &&
         chk(bioem_b200_synchronize(h), "synchronize");
     handles[g] = h;

@@ -59,6 +59,10 @@ static void usage()
          "                         file, one MRC mode-2 stack that --ReadMRC with NO_MAP_NORM reads back as the\n"
          "                         rendered images.  Not the reference's --PrintBestCalMap: its parameter keywords,\n"
          "                         BESTMAP text format and noise option are not reproduced\n"
+         "  --DefocusPerParticle arg (Extension) file with one defocus [micro-m] per particle, in particle order:\n"
+         "                         particles with equal values form one CTF group, whose defocus grid has\n"
+         "                         CTF_DEFOCUS's width and count centred on the value, and whose PRIOR_DEFOCUS_CENTER\n"
+         "                         is the value; every particle integrates over its own group's CTFs only\n"
          "  --help                 (Optional) Produce help message\n\n");
 }
 
@@ -111,6 +115,8 @@ void parse_options(int argc, char **argv, Options &o)
       o.gpus = atoi(need().c_str());
     else if (a == "WriteBestMaps")
       o.bestmapsfile = need();
+    else if (a == "DefocusPerParticle")
+      o.defocusfile = need();
     else if (a == "ReadPDB")
       o.readPDB = true;
     else if (a == "ReadModelMRC")
@@ -393,6 +399,8 @@ void read_parameters(const std::string &file, Params &p)
       fail("Input missing: please provide grid CTF defocus");
     if (!yAmp)
       fail("Input missing: please provide grid CTF amplitude");
+    p.startDef = startDef;
+    p.endDef = endDef;
     // defocus [micro-m] -> phase, prior centre and width scaled alike (param.cpp:601-607)
     bioem_b200_host_defocus_to_phase(startDef, endDef, p.elecwavel, &p.startPhase, &p.endPhase, &p.Priordefcent,
                                      &p.sigmaPriordefo);
@@ -566,6 +574,80 @@ void make_ctf_table(Params &p)
   }
   p.volu = bioem_b200_host_volu(p.voluang, p.GridSpaceCenter, p.pixelSize, p.maxDisplaceCenter, p.nAmp, grids[2], grids[1],
                                 p.sigmaPriorbctf, p.sigmaPriordefo, p.sigmaPrioramp);
+}
+
+void make_ctf_groups(const std::string &file, int nMaps, Params &p)
+{
+  if (p.usepsf)
+    fail("--DefocusPerParticle: USE_PSF kernels are complex; CTF groups need CTF_DEFOCUS tables");
+  std::ifstream in(file.c_str());
+  if (!in.good())
+    fail("--DefocusPerParticle: cannot open %s", file.c_str());
+  std::vector<float> vals;
+  std::string tok;
+  while (in >> tok)
+  {
+    char *end = nullptr;
+    const float v = strtof(tok.c_str(), &end);
+    if (end == tok.c_str() || *end != 0)
+      fail("--DefocusPerParticle %s: entry %d (%s) is not a number", file.c_str(), (int) vals.size(), tok.c_str());
+    vals.push_back(v);
+  }
+  if ((int) vals.size() != nMaps)
+    fail("--DefocusPerParticle %s: %d values for %d particles", file.c_str(), (int) vals.size(), nMaps);
+  std::vector<float> defs; // one per group, in order of first appearance
+  p.group.assign(nMaps, 0);
+  for (int m = 0; m < nMaps; m++)
+  {
+    const auto it = std::find(defs.begin(), defs.end(), vals[m]);
+    p.group[m] = (int) (it - defs.begin());
+    if (it == defs.end())
+      defs.push_back(vals[m]);
+  }
+  const int G = (int) defs.size();
+  const float half = 0.5f * (p.endDef - p.startDef);
+  const size_t F = (size_t) p.N * (p.N / 2 + 1);
+  std::vector<float> ref, par;
+  p.groupDefcent.assign(G, 0.f);
+  float volu0 = 0.f;
+  int C = 0;
+  for (int g = 0; g < G; g++)
+  {
+    const float d0 = defs[g] - half, d1 = defs[g] + half;
+    // the reference's checks of CTF_DEFOCUS (param.cpp), per group
+    if (d0 < 0)
+      fail("--DefocusPerParticle: defocus %g: Negative start defocus (%g)", (double) defs[g], (double) d0);
+    if (d1 > 8.)
+      fail("--DefocusPerParticle: defocus %g: Defocus beyond 8micro-m range is not allowed (%g)", (double) defs[g],
+           (double) d1);
+    float ph0, ph1, cen = defs[g];
+    bioem_b200_host_defocus_to_phase(d0, d1, p.elecwavel, &ph0, &ph1, &cen, nullptr);
+    float grids[3];
+    const int c = bioem_b200_host_ctf_table(p.N, p.pixelSize, 0, p.startAmp, p.endAmp, p.nAmp, ph0, ph1, p.nPhase, p.startEnv,
+                                            p.endEnv, p.nEnv, nullptr, nullptr, grids);
+    if (c <= 0 || (g > 0 && c != C))
+      fail("--DefocusPerParticle: defocus %g: CTF grid of %d kernels", (double) defs[g], c);
+    C = c;
+    ref.resize((size_t) (g + 1) * C * F * 2);
+    par.resize((size_t) (g + 1) * C * 4);
+    bioem_b200_host_ctf_table(p.N, p.pixelSize, 0, p.startAmp, p.endAmp, p.nAmp, ph0, ph1, p.nPhase, p.startEnv, p.endEnv,
+                              p.nEnv, &ref[(size_t) g * C * F * 2], &par[(size_t) g * C * 4], grids);
+    // every group has the grid steps of CTF_DEFOCUS, so the same volu (up to the rounding of the phase step)
+    const float volu = bioem_b200_host_volu(p.voluang, p.GridSpaceCenter, p.pixelSize, p.maxDisplaceCenter, p.nAmp, grids[2],
+                                            grids[1], p.sigmaPriorbctf, p.sigmaPriordefo, p.sigmaPrioramp);
+    if (g == 0)
+      volu0 = volu;
+    else if (!(fabsf(volu - volu0) <= 1e-5f * fabsf(volu0)))
+      fail("--DefocusPerParticle: defocus %g: volume element %g differs from the first group's %g", (double) defs[g],
+           (double) volu, (double) volu0);
+    p.groupDefcent[g] = cen;
+  }
+  p.refCTF.swap(ref);
+  p.CtfParam.swap(par);
+  p.nCtf = C;
+  p.nGroups = G;
+  p.volu = volu0;
+  std::cout << "CTF groups: " << G << " defocus values, " << C << " CTF kernels each\n";
 }
 
 // --------------------------------------------------------------------------- MRC helpers

@@ -115,6 +115,24 @@ int bioem_b200_upload_ctf(bioem_b200_handle h, const float *refCTF, const float 
 /* USE_PSF: the nCtf kernels given as real-space point-spread functions (nCtf x N x N); the library
  * takes their forward r2c transform, which the reference does on the host (param.cpp:1466-1535). */
 int bioem_b200_upload_ctf_real(bioem_b200_handle h, const float *kernels, const float *CtfParam4, int nCtf);
+/* Per-micrograph CTF groups: G tables of C rows each, group-major (G*C rows in the layouts of upload_ctf), and
+ * Priordefcent[G], each group's defocus-prior centre in phase units (NULL: the config's Priordefcent for all).  Row
+ * g*C + c's prior is that of upload_ctf with group g's centre.  After set_particle_groups, particle m integrates over
+ * the C rows of its own group only, and every record names a row of the whole table (max_prob_conv = g*C + c), so
+ * render_maps, download and the multi-GPU merges need no knowledge of groups.  A grouped run gives what G separate
+ * ungrouped runs (group g's table, group g's particles) give: the same records and angle rows; Total bit for bit at
+ * the same batch geometry (BIOEM_B200_OB / BIOEM_B200_OG), else up to the order of the partial merges.  The table
+ * must be real (CTFs computed in Fourier space: cached-product mode, which a grouped table always runs in).  Refused
+ * (BIOEM_B200_ERR_INVALID): a non-zero imaginary part, USE_PSF, G < 1, C < 1, and an edge without a fused kernel
+ * (bioem_b200_supported_size(N) == 0); run() refuses BIOEM_B200_CACHED_PRODUCT=0 with it.  debug_run_values captures
+ * [o][c][m] with c < C (each particle's own rows).  upload_ctf / upload_ctf_real replace a grouped table by an
+ * ungrouped one and drop the particle groups; a new grouped table keeps them while they name groups it has. */
+int bioem_b200_upload_ctf_groups(bioem_b200_handle h, const float *refCTF, const float *CtfParam4, const float *Priordefcent,
+                                 int G, int C);
+/* group[nMaps]: the CTF group of every particle, in [0, G).  nMaps must be the uploaded particle count; needs the
+ * particles and a grouped table on the handle (else BIOEM_B200_ERR_STATE).  Invalidates the running state like an
+ * upload; upload_particles* drop the list.  run() with a grouped table and no list returns BIOEM_B200_ERR_STATE. */
+int bioem_b200_set_particle_groups(bioem_b200_handle h, const int *group, int nMaps);
 /* RefMap.maps (nMaps x N x N, as read, BEFORE RefMap.precalculate): the library
  * computes sum_RefMap / sumsquare_RefMap / RefMapsFFT itself (replaces reference
  * map.cpp:557-630). */
